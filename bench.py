@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - reads/s of Shark's k-mer Bloom-filter hot path on B200 (see DESIGN.md, Measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workloads c4,c3,c2]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workloads c4,c3,c2] [--dump-outputs DIR]
 
 A step = one pass of the hot path over this rank's whole batch of synthetic reads.
   N = 1   the default run measures C4 (headline: the largest single-GPU configuration of BASELINE.json - 20 k genes,
@@ -55,6 +55,7 @@ WORKLOADS = {
                     "index replicated (NCCL broadcast; also built by the sharded P2P OR-merge mode)"),
 }
 CHUNK_READS = 1 << 20
+DUMP_BYTES = 64_000_000   # --dump-outputs: all files together
 REF_BIN = os.path.join(ROOT, "oracle", "_ref", "shark")
 CLI_BIN = os.path.join(ROOT, "shark_b200", "shark-b200")
 
@@ -146,6 +147,32 @@ def traffic_for(name):
     if t.get("kernel_source_hash") != kernel_source_hash():
         return None, "the ncu capture on file is of other kernel sources (%s): not reported" % t.get("kernel_source_hash")
     return t.get("dram_bytes_per_launch"), t.get("source")
+
+
+def dump_outputs(outdir, prefix, outputs, budget):
+    """Writes what one step of the value leg returned, expanded as a caller of the API receives it (Shark.expand: per
+    read the gene16 code, 0xFFFF none and 0xFFFE several, and the (read, gene) associations), as three arrays over the
+    rank's reads:
+      <prefix>_read.npy   float64[m]     indices of the reads written (all reads, or a fixed seeded sample when all of
+                                         them would not fit in `budget` bytes)
+      <prefix>_gene.npy   float32[m]     gene16 of those reads
+      <prefix>_assoc.npy  float64[r, 2]  (read, gene) associations of those reads, by read then gene"""
+    from shark_b200.engine import Shark
+    gene, assoc, first = [], [], 0
+    for g, m in outputs:
+        ridx, gidx, _ = Shark.expand({"gene16": g, "multi": m})
+        gene.append(g)
+        assoc.append(np.stack([ridx.astype(np.int64) + first, gidx.astype(np.int64)], 1))
+        first += len(g)
+    gene, assoc = np.concatenate(gene), np.concatenate(assoc)
+    n = len(gene)
+    m = min(n, (budget - 1024) // 24)   # 12 bytes per read written; at least as much is left for the associations
+    reads = np.arange(n) if m == n else np.sort(np.random.default_rng(0).choice(n, m, replace=False))
+    rows = assoc[np.isin(assoc[:, 0], reads)][: (budget - 1024 - 12 * m) // 16]
+    os.makedirs(outdir, exist_ok=True)
+    for key, a in (("read", reads.astype(np.float64)), ("gene", gene[reads].astype(np.float32)),
+                   ("assoc", rows.astype(np.float64))):
+        np.save(os.path.join(outdir, "%s_%s.npy" % (prefix, key)), a)
 
 
 def probe_kmers(bases, k, n, seed=7):
@@ -561,13 +588,16 @@ def run_workload(name, args, rank, world, local_rank, cores, dist, torch):
         sh.timer_start()  # device stopwatch (CUDA events over all slot streams); the host clock is the cross-check
         tot = dict(n_probes=0, n_hits=0, n_assoc=0, n_slow_reads=0, n_extended=0, n_table_loads=0, n_multi=0, n_kept=0)
         for _ in range(args.steps):
-            for r in step():
+            last = step()
+            for r in last:
                 for key in tot:
                     tot[key] += r[key]
         t_dev = sh.timer_stop() * 1e-3
         barrier()
         t_wall = time.perf_counter() - t0
         launches = sh.kernel_launches() - l0
+        # the last timed step's results, copied before the roofline pass below overwrites the slots' result buffers
+        outputs = [(r["gene16"].copy(), r["multi"].copy()) for r in last] if args.dump_outputs else None
         # roofline pass: the same launches one at a time (no overlap between the slots' streams), so that the
         # CUDA-event time of analyze_reads_kernel is the time of that kernel alone
         probe_ms = 0.0
@@ -575,7 +605,7 @@ def run_workload(name, args, rank, world, local_rank, cores, dist, torch):
             for i in range(n_chunks):
                 sh.analyze_resident(i)
                 probe_ms += sh.collect(i, copy=False)["probe_kernel_ms"]
-        return dict(t_dev=t_dev, t_wall=t_wall, launches=launches, probe_ms=probe_ms, **tot)
+        return dict(t_dev=t_dev, t_wall=t_wall, launches=launches, probe_ms=probe_ms, outputs=outputs, **tot)
 
     sampler = ClockSampler(local_rank)
     sampler.start()
@@ -672,6 +702,8 @@ def run_workload(name, args, rank, world, local_rank, cores, dist, torch):
     t_value = t_packed if value_form == "packed" else t_text
     res_v = res_packed if value_form == "packed" else res_text
     roofline = roofline_of(res_v, pm_packed if value_form == "packed" else pm_text, value_form)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, name if world == 1 else "%s_rank%d" % (name, rank), res_v["outputs"], args.dump_bytes)
 
     # ---- parity
     cpu_baseline, parity_ranks = None, None
@@ -808,6 +840,9 @@ def main():
     ap.add_argument("--value-form", default="packed", choices=["text", "packed"],
                     help="form in which the reads are resident in HBM for `value` (both are measured: value_by_form)")
     ap.add_argument("--e2e-slots", type=int, default=5, help="chunks in flight in the e2e legs")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="after the timed steps, write what the last one returned for every workload as DIR/<workload>_"
+                         "{read,gene,assoc}.npy (float, at most 64 MB in all), so that two builds can be compared")
     ap.add_argument("--index", default="", choices=["", "broadcast", "sharded", "both"],
                     help="N > 1: build on rank 0 + NCCL broadcast, the sharded P2P OR-merge build, or both (default) with an "
                          "equality check on every rank")
@@ -820,6 +855,11 @@ def main():
     for w in names:
         if w not in WORKLOADS:
             raise SystemExit("unknown workload %r" % w)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes what this project computes; the reference arm computes nothing of ours")
+    args.dump_bytes = DUMP_BYTES // (len(names) * world)   # every workload and rank gets an equal share
     head = WORKLOADS[names[0]]
 
     # ---------------------------------------------------------------- reference arm

@@ -5,7 +5,8 @@ built by oracle/Makefile from /root/reference) on
   example/   the reference's own fixture (example/ENSG00000277117.fa, sample_{1,2}.fq; inputs
              stored gzipped, the three truth files stored as md5 + gz) under the flag
              variants of SURVEY.md App. B.2, and
-  edge/      small generated inputs, one scenario per quirk of SURVEY.md App. C.
+  edge/      small generated inputs, one scenario per quirk of SURVEY.md App. C, and
+  synth/     the larger generated inputs of tests/test_cli.py, kept as digests of the outputs.
 
 Run here (needs /root/reference); the outputs are committed so the GPU box needs neither.
     python tests/golden/make_golden.py
@@ -241,7 +242,38 @@ def make_edge():
     json.dump(index, open(os.path.join(d, "cases.json"), "w"), indent=1, sort_keys=True)
 
 
+# ---------------------------------------------------------------------------------------
+SYNTH = {   # generated inputs of tests/test_cli.py: pairs, read length, seed of the reads, flag variants
+    "pairs": (120000, 75, 11, {"k17": ["-k", "17"], "k21_q20_s": ["-k", "21", "-q", "20", "-s"],
+                               "k31_c0.8_b2": ["-k", "31", "-c", "0.8", "-b", "2"]}),
+    "bgzf": (150000, 100, 13, {"k21_q20": ["-k", "21", "-q", "20"]}),
+}
+
+
+def make_synth():
+    """synth/cases.json: the reference's help text, and digests of what it prints and writes for generated inputs
+    (tests/helpers.py stage_synth) too large to store."""
+    sys.path[:0] = [ROOT, os.path.join(ROOT, "tests")]
+    from helpers import stage_synth
+    d = os.path.join(HERE, "synth")
+    os.makedirs(d, exist_ok=True)
+    out = {"help": subprocess.run([REF_BIN, "-h"], stdout=subprocess.PIPE, stderr=subprocess.PIPE).stderr.decode()}
+    for key, (n, read_len, seed, cases) in SYNTH.items():
+        with tempfile.TemporaryDirectory() as tmp:
+            files = stage_synth(tmp, n, read_len, seed)
+            res = {}
+            for name, flags in cases.items():
+                o = run_ref("ref.fa", "a_1.fq", "a_2.fq", flags, tmp)
+                res[name] = {"flags": flags, "rc": o["rc"], "ssv_lines": o["ssv"].count(b"\n"), "ssv_md5": md5(o["ssv"]),
+                             "o1_md5": md5(o["o1"]), "o2_md5": md5(o["o2"])}
+                print("synth", key, name, res[name]["ssv_lines"], file=sys.stderr)
+            out[key] = {"pairs": n, "read_len": read_len, "seed": seed, "cases": res,
+                        "inputs_md5": {f: md5(open(p, "rb").read()) for f, p in files.items()}}
+    json.dump(out, open(os.path.join(d, "cases.json"), "w"), indent=1, sort_keys=True)
+
+
 if __name__ == "__main__":
     assert os.path.exists(REF_BIN), "build the reference first: make -C oracle ref"
     make_example()
     make_edge()
+    make_synth()

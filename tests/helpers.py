@@ -33,6 +33,22 @@ def edge_cases():
     return json.load(open(os.path.join(GOLDEN, "edge", "cases.json")))
 
 
+def synth_cases():
+    return json.load(open(os.path.join(GOLDEN, "synth", "cases.json")))
+
+
+def stage_synth(tmpdir, n_pairs, read_len, seed):
+    """ref.fa (60 generated genes) and a_1.fq / a_2.fq (n_pairs generated read pairs with varied qualities) in tmpdir;
+    the same bytes on every machine, so that what the reference printed for them can be stored as digests."""
+    from shark_b200 import synth
+    names, bases, rec_off = synth.make_reference(60, seed=7)
+    synth.write_fasta(os.path.join(str(tmpdir), "ref.fa"), names, bases, rec_off)
+    seq, qual, _ = synth.make_reads(bases, 60, n_pairs, read_len, True, seed=seed, varied_qual=True, want_qual=True)
+    synth.write_fastq(os.path.join(str(tmpdir), "a_1.fq"), os.path.join(str(tmpdir), "a_2.fq"), seq, qual, n_pairs,
+                      read_len, True)
+    return {f: os.path.join(str(tmpdir), f) for f in ("ref.fa", "a_1.fq", "a_2.fq")}
+
+
 def flags_to_kwargs(flags):
     """['-k','31','-s'] -> dict(k=31, single=True, ...) (argument_parser.hpp:84-174 defaults)."""
     kw = dict(k=17, c=0.6, b=1, q=0, single=False)

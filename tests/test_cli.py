@@ -5,7 +5,7 @@ import subprocess
 
 import pytest
 
-from helpers import GOLDEN, ROOT, edge_cases, example_cases, gz_read, md5, stage_edge, stage_example
+from helpers import GOLDEN, ROOT, edge_cases, example_cases, gz_read, md5, stage_edge, stage_example, stage_synth, synth_cases
 
 CLI = os.path.join(ROOT, "shark_b200", "shark-b200")
 REF = os.path.join(ROOT, "oracle", "_ref", "shark")
@@ -46,7 +46,7 @@ def test_argument_errors_match_reference(tmp_path, args, msg):
 
 def test_help_matches_reference(tmp_path):
     rc, out, err = run_cli(["-h"], tmp_path)
-    assert rc == 0 and out == b"" and err.startswith(b"Usage: shark -r <references> -1 <sample1>")
+    assert rc == 0 and out == b"" and err.decode() == synth_cases()["help"]
     if os.path.exists(REF):
         assert run_cli(["-h"], tmp_path, exe=REF) == (rc, out, err)
 
@@ -114,25 +114,38 @@ def test_cli_gz_inputs_small_chunks_and_default_outputs(tmp_path):
     assert b"[shark/Sample completed] Time elapsed" in err
 
 
+def _stage_synth_set(tmp_path, s):
+    f = stage_synth(tmp_path, s["pairs"], s["read_len"], s["seed"])
+    assert {k: md5(open(p, "rb").read()) for k, p in f.items()} == s["inputs_md5"], "shark_b200.synth generates other inputs"
+    return f
+
+
+def test_synth_inputs_are_the_ones_of_the_goldens(tmp_path):
+    """tests/golden/synth holds what the reference printed for generated inputs: they must still be generated the same."""
+    for s in ("pairs", "bgzf"):
+        _stage_synth_set(tmp_path, synth_cases()[s])
+
+
 @pytest.mark.gpu
 def test_cli_against_live_reference_binary(tmp_path):
-    """A fresh random input run through both binaries on this box (skipped when the compiled
-    reference did not travel)."""
-    if not os.path.exists(REF):
-        pytest.skip("oracle/_ref/shark not present")
-    import numpy as np
-    from shark_b200 import synth
-    names, bases, rec_off = synth.make_reference(60, seed=7)
-    synth.write_fasta(str(tmp_path / "ref.fa"), names, bases, rec_off)
-    seq, qual, _ = synth.make_reads(bases, 60, 120000, 75, True, seed=11, varied_qual=True, want_qual=True)
-    synth.write_fastq(str(tmp_path / "a_1.fq"), str(tmp_path / "a_2.fq"), seq, qual, 120000, 75, True)
-    for flags in (["-k", "17"], ["-k", "21", "-q", "20", "-s"], ["-k", "31", "-c", "0.8", "-b", "2"]):
+    """A fresh random input through the CLI: byte for byte what the reference binary printed and wrote for it
+    (digests in tests/golden/synth), and what the binary itself does when oracle/_ref/shark is built."""
+    s = synth_cases()["pairs"]
+    _stage_synth_set(tmp_path, s)
+    for info in s["cases"].values():
+        flags = info["flags"]
         base = ["-r", "ref.fa", "-1", "a_1.fq", "-2", "a_2.fq"]
         rc, out, err = run_cli(base + ["-o", "m1.fq", "-p", "m2.fq"] + flags, tmp_path)
-        assert rc == 0, err.decode()
+        assert rc == info["rc"] == 0, err.decode()
+        assert out.count(b"\n") == info["ssv_lines"] and len(out) > 1000
+        assert md5(out) == info["ssv_md5"]
+        assert md5(open(str(tmp_path / "m1.fq"), "rb").read()) == info["o1_md5"]
+        assert md5(open(str(tmp_path / "m2.fq"), "rb").read()) == info["o2_md5"]
+        if not os.path.exists(REF):
+            continue
         rc0, out0, err0 = run_cli(base + ["-o", "r1.fq", "-p", "r2.fq"] + flags, tmp_path, exe=REF)
         assert rc0 == 0
-        assert out == out0 and len(out) > 1000
+        assert out == out0
         for a, b in (("m1.fq", "r1.fq"), ("m2.fq", "r2.fq")):
             assert open(str(tmp_path / a), "rb").read() == open(str(tmp_path / b), "rb").read()
 
@@ -141,21 +154,17 @@ def test_cli_against_live_reference_binary(tmp_path):
 def test_cli_blocked_gzip_inputs_parallel_inflate(tmp_path):
     """Samples compressed as BGZF (bgzip): the CLI inflates the blocks in parallel (`-t 4` = four inflate threads per
     file + read-ahead, csrc/host/bgzf.hpp) and must print what it prints for the plain files - and what the reference
-    prints when it reads the very same .gz files through gzread."""
+    prints when it reads the very same .gz files through gzread (digests in tests/golden/synth)."""
     import random
     from test_host_ingest import _bgzf
-    import numpy as np
-    from shark_b200 import synth
-    names, bases, rec_off = synth.make_reference(60, seed=7)
-    synth.write_fasta(str(tmp_path / "ref.fa"), names, bases, rec_off)
-    n = 150000
-    seq, qual, _ = synth.make_reads(bases, 60, n, 100, True, seed=13, varied_qual=True, want_qual=True)
-    synth.write_fastq(str(tmp_path / "a_1.fq"), str(tmp_path / "a_2.fq"), seq, qual, n, 100, True)
+    s = synth_cases()["bgzf"]
+    _stage_synth_set(tmp_path, s)
     rng = random.Random(3)
     for m in ("1", "2"):
         data = open(str(tmp_path / ("a_%s.fq" % m)), "rb").read()
         open(str(tmp_path / ("a_%s.fq.gz" % m)), "wb").write(b"".join(_bgzf(data, rng)))
-    flags = ["-k", "21", "-q", "20"]
+    info = s["cases"]["k21_q20"]
+    flags = info["flags"]
     rc, out, err = run_cli(["-r", "ref.fa", "-1", "a_1.fq", "-2", "a_2.fq", "-o", "p1.fq", "-p", "p2.fq"] + flags, tmp_path)
     assert rc == 0, err.decode()
     rc, outz, err = run_cli(["-r", "ref.fa", "-1", "a_1.fq.gz", "-2", "a_2.fq.gz", "-o", "z1.fq", "-p", "z2.fq", "-t", "4",
@@ -164,6 +173,9 @@ def test_cli_blocked_gzip_inputs_parallel_inflate(tmp_path):
     assert outz == out and len(out) > 100000
     for a, b in (("z1.fq", "p1.fq"), ("z2.fq", "p2.fq")):
         assert open(str(tmp_path / a), "rb").read() == open(str(tmp_path / b), "rb").read()
+    assert (md5(out), out.count(b"\n")) == (info["ssv_md5"], info["ssv_lines"])
+    assert md5(open(str(tmp_path / "z1.fq"), "rb").read()) == info["o1_md5"]
+    assert md5(open(str(tmp_path / "z2.fq"), "rb").read()) == info["o2_md5"]
     if os.path.exists(REF):
         rc0, out0, _ = run_cli(["-r", "ref.fa", "-1", "a_1.fq.gz", "-2", "a_2.fq.gz", "-o", "r1.fq", "-p", "r2.fq"] + flags,
                                tmp_path, exe=REF)

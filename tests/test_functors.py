@@ -1,10 +1,11 @@
 """The reference's functor seam (SURVEY.md 8b, seam 2): KmerBuilder / BloomfilterFiller / class BF /
 ReadAnalyzer re-implemented over the C ABI (include/shark_b200_functors.hpp, the staged shk_bf_* calls).
 
-CPU: the header compiles stand-alone, and the reference's own main.cpp built on top of it
-(oracle/_ref/shark_hybrid) fails loudly without a device.
+CPU: the header compiles stand-alone, and the hybrid executable fails loudly without a device.
 GPU: every staged call against the oracle, the protocol end to end against the one-call build, and the
-hybrid executable byte-for-byte against the reference's goldens."""
+hybrid executable byte-for-byte against the reference's goldens.
+The hybrid executable is the reference's own main.cpp built on the header (oracle/_ref/shark_hybrid) where that has
+been built, and otherwise tests/host_tools/functor_main.cpp, a restatement of that driver on the same header."""
 import os
 import subprocess
 
@@ -13,7 +14,7 @@ import pytest
 
 from helpers import GOLDEN, ROOT, edge_cases, example_cases, gz_read, md5, stage_edge, stage_example
 
-HYBRID = os.path.join(ROOT, "oracle", "_ref", "shark_hybrid")
+REF_HYBRID = os.path.join(ROOT, "oracle", "_ref", "shark_hybrid")
 REF = os.path.join(ROOT, "oracle", "_ref", "shark")
 
 
@@ -23,6 +24,19 @@ def _built():
     build.build()
     from oracle import pyoracle
     pyoracle.build()
+
+
+@pytest.fixture(scope="module")
+def hybrid(tmp_path_factory):
+    if os.path.exists(REF_HYBRID):
+        return REF_HYBRID
+    out = str(tmp_path_factory.mktemp("hybrid") / "functor_main")
+    lib = os.path.join(ROOT, "shark_b200")
+    subprocess.check_call(["g++", "-O2", "-std=c++14", "-Wall", "-I", os.path.join(ROOT, "include"), "-I",
+                           os.path.join(ROOT, "tests", "host_tools"), os.path.join(ROOT, "tests", "host_tools", "functor_main.cpp"),
+                           "-o", out, "-L", lib, "-lshark_b200", "-Wl,-rpath," + lib, "-Wl,-rpath-link,/usr/local/cuda/lib64",
+                           "-lz", "-pthread"])
+    return out
 
 
 # ------------------------------------------------------------------------------------------- CPU
@@ -43,14 +57,12 @@ def test_functor_header_compiles_standalone(tmp_path):
                    check=True)
 
 
-def test_hybrid_fails_loudly_without_gpu(tmp_path):
+def test_hybrid_fails_loudly_without_gpu(tmp_path, hybrid):
     import torch
     if torch.cuda.is_available():
         pytest.skip("a GPU is present")
-    if not os.path.exists(HYBRID):
-        pytest.skip("oracle/_ref/shark_hybrid is not built (needs /root/reference)")
     f = stage_example(tmp_path)
-    p = subprocess.run([HYBRID, "-r", f["ENSG00000277117.fa"], "-1", f["sample_1.fq"]], cwd=str(tmp_path),
+    p = subprocess.run([hybrid, "-r", f["ENSG00000277117.fa"], "-1", f["sample_1.fq"]], cwd=str(tmp_path),
                        stdout=subprocess.PIPE, stderr=subprocess.PIPE)
     assert p.returncode == 1 and p.stdout == b"" and b"no CUDA device" in p.stderr
 
@@ -209,11 +221,9 @@ def _run(exe, args, cwd):
     return p.returncode, p.stdout, p.stderr
 
 
-def _hybrid_case(tmp_path, ref, s1, s2, flags):
-    if not os.path.exists(HYBRID):
-        pytest.skip("oracle/_ref/shark_hybrid did not travel")
+def _hybrid_case(hybrid, tmp_path, ref, s1, s2, flags):
     args = ["-r", ref, "-1", s1, "-o", "o1.fq"] + (["-2", s2, "-p", "o2.fq"] if s2 else []) + list(flags)
-    rc, out, err = _run(HYBRID, args, tmp_path)
+    rc, out, err = _run(hybrid, args, tmp_path)
     assert rc == 0, err.decode()
     o1 = open(os.path.join(str(tmp_path), "o1.fq"), "rb").read()
     o2 = open(os.path.join(str(tmp_path), "o2.fq"), "rb").read() if s2 else None
@@ -222,11 +232,11 @@ def _hybrid_case(tmp_path, ref, s1, s2, flags):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("case", sorted(example_cases()["cases"]))
-def test_hybrid_example_goldens(tmp_path, case):
+def test_hybrid_example_goldens(tmp_path, hybrid, case):
     """The reference's main.cpp + our functors reproduce the reference's own truth files."""
     info = example_cases()["cases"][case]
     f = stage_example(tmp_path)
-    ssv, o1, o2 = _hybrid_case(tmp_path, f["ENSG00000277117.fa"], f["sample_1.fq"],
+    ssv, o1, o2 = _hybrid_case(hybrid, tmp_path, f["ENSG00000277117.fa"], f["sample_1.fq"],
                                f["sample_2.fq"] if info["paired"] else None, info["flags"])
     assert (md5(ssv), md5(o1)) == (info["ssv_md5"], info["o1_md5"])
     if info["paired"]:
@@ -235,10 +245,10 @@ def test_hybrid_example_goldens(tmp_path, case):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("scenario,case", [(s, c) for s, cs in sorted(edge_cases().items()) for c in sorted(cs)])
-def test_hybrid_edge_goldens(tmp_path, scenario, case):
+def test_hybrid_edge_goldens(tmp_path, hybrid, scenario, case):
     info = edge_cases()[scenario][case]
     f = stage_edge(tmp_path, scenario)
-    ssv, o1, o2 = _hybrid_case(tmp_path, f["ref.fa"], f["r1.fq"], f.get("r2.fq") if info["paired"] else None, info["flags"])
+    ssv, o1, o2 = _hybrid_case(hybrid, tmp_path, f["ref.fa"], f["r1.fq"], f.get("r2.fq") if info["paired"] else None, info["flags"])
     d = os.path.join(GOLDEN, "edge", scenario)
     assert ssv == gz_read(os.path.join(d, case + ".ssv.gz"))
     assert o1 == gz_read(os.path.join(d, case + ".o1.fq.gz"))
@@ -250,7 +260,7 @@ def test_hybrid_edge_goldens(tmp_path, scenario, case):
 def test_hybrid_threads_against_live_reference(tmp_path):
     """-t 4: ReadAnalyzer::operator() is called concurrently (main.cpp:219-223); the set of output
     lines and of kept records equals the reference binary's (Q12: only the order may differ)."""
-    if not (os.path.exists(HYBRID) and os.path.exists(REF)):
+    if not (os.path.exists(REF_HYBRID) and os.path.exists(REF)):
         pytest.skip("compiled reference binaries did not travel")
     from shark_b200 import synth
     names, bases, rec_off = synth.make_reference(80, seed=5)
@@ -264,7 +274,7 @@ def test_hybrid_threads_against_live_reference(tmp_path):
 
     for flags in (["-k", "17", "-t", "4"], ["-k", "21", "-q", "20", "-s", "-t", "3"]):
         base = ["-r", "ref.fa", "-1", "a_1.fq", "-2", "a_2.fq"]
-        rc, out, err = _run(HYBRID, base + ["-o", "h1.fq", "-p", "h2.fq"] + flags, tmp_path)
+        rc, out, err = _run(REF_HYBRID, base + ["-o", "h1.fq", "-p", "h2.fq"] + flags, tmp_path)
         assert rc == 0, err.decode()
         rc0, out0, _ = _run(REF, base + ["-o", "r1.fq", "-p", "r2.fq"] + flags, tmp_path)
         assert rc0 == 0 and len(out0) > 1000
