@@ -85,6 +85,10 @@ typedef struct shk_params {
  * (warp per read), results arrive through the `multi` list, and the staged functor protocol
  * (shk_bf_add_to_kmer) is not available. */
 #define SHK_F_WIDE_IDS 16u
+/* Keep a score record per read (shk_read_score, shk_reads_scores): the numbers behind each read's yes/no answer,
+ * so that a caller can classify a sample once and apply any -c and -s afterwards (INTEGRATION.md 3).  16 bytes per
+ * read more cross the link; without the flag nothing is written, allocated or copied. */
+#define SHK_F_SCORES 32u
 
 /* Compact per-read result words (shk_chunk_result.gene16). */
 #define SHK_GENE_NONE 0xFFFFu  /* no association: the read is not reported                                */
@@ -156,6 +160,22 @@ typedef struct shk_chunk_result {
 /* Expands a compact result into the association list (n_assoc entries) and the keep flags (n_reads); either
  * output may be NULL.  Pure host function. */
 int shk_result_expand(const shk_chunk_result *result, shk_assoc *assoc, uint8_t *keep);
+
+/* The numbers behind one read's answer (SHK_F_SCORES).  A read is reported iff
+ *     n_best > 0  &&  (double)cov >= c * len  &&  (!single || n_best == 1)
+ * (c * len the IEEE double product, ReadAnalyzer.hpp:104), and a reported read has exactly n_best associations.
+ * None of the four depends on c or -s: a run at c = 0 without -s, filtered by this rule, gives the run at any
+ * (c, -s) association for association. */
+typedef struct shk_read_score {
+    uint32_t len;    /* valid bases after the -q masking: ReadAnalyzer's len (ReadAnalyzer.hpp:46-49)              */
+    uint32_t cov;    /* coverage of the best gene (`max`, ReadAnalyzer.hpp:90-102); 0 if no gene was hit           */
+    uint32_t hits;   /* k-mer hits of the best gene (`maxk`); 0 if no gene was hit                                 */
+    uint32_t n_best; /* genes tied at (cov, hits), BEFORE the threshold and -s; 0 if no gene was hit              */
+} shk_read_score;
+/* After shk_reads_collect(slot): n_reads records, one per read of the chunk in read order, in library-owned pinned
+ * memory, valid until the slot's next submit (same lifetime as gene16).  A read without a window of k valid bases
+ * gets {len, 0, 0, 0}.  SHK_E_STATE for a context created without SHK_F_SCORES or before the slot is collected. */
+int shk_reads_scores(shk_ctx *ctx, uint32_t slot, const shk_read_score **scores, uint32_t *n_reads);
 
 /* ---- lifetime ------------------------------------------------------------------------ */
 
@@ -387,7 +407,7 @@ int shk_upload_stats(const shk_ctx *ctx, double *packed_share, double *pack_gbas
 
 /* Bytes that shk_reads_submit / shk_reads_upload copied host -> device on this context so far. */
 uint64_t shk_h2d_bytes(const shk_ctx *ctx);
-/* Result bytes (associations, keep flags, counters) copied device -> host on this context so far.  The
+/* Result bytes (associations, keep flags, counters, score records) copied device -> host on this context so far.  The
  * read-back of a chunk is enqueued with its kernels, sized by the previous chunks' associations per read;
  * shk_reads_collect fetches what that did not cover. */
 uint64_t shk_d2h_bytes(const shk_ctx *ctx);

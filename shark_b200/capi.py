@@ -25,7 +25,7 @@ EXPORTED = [
     "shk_set_options", "shk_shard_begin", "shk_shard_open", "shk_shard_close", "shk_shard_merge", "shk_shard_rank",
     "shk_shard_finish", "shk_shard_end", "shk_shard_cuts", "shk_index_build_sharded", "shk_index_save", "shk_index_load",
     "shk_host_pack", "shk_host_pack_info", "shk_h2d_bytes", "shk_d2h_bytes", "shk_set_upload_mode", "shk_upload_stats",
-    "shk_reads_submit_packed", "shk_reads_upload_packed", "shk_result_expand", "shk_index_export_wide",
+    "shk_reads_submit_packed", "shk_reads_upload_packed", "shk_result_expand", "shk_index_export_wide", "shk_reads_scores",
 ]
 
 
@@ -42,7 +42,7 @@ class Params(C.Structure):
                 ("host_pack_permille", C.c_uint32), ("reserved", C.c_uint32 * 6)]
 
 
-F_EXTEND_ON, F_EXTEND_OFF, F_HOST_PACK, F_COMPACT_RESULTS, F_WIDE_IDS = 1, 2, 4, 8, 16
+F_EXTEND_ON, F_EXTEND_OFF, F_HOST_PACK, F_COMPACT_RESULTS, F_WIDE_IDS, F_SCORES = 1, 2, 4, 8, 16, 32
 GENE_NONE, GENE_MULTI = 0xFFFF, 0xFFFE
 
 
@@ -66,6 +66,11 @@ class IndexViews(C.Structure):
 
 class Assoc(C.Structure):
     _fields_ = [("read_idx", C.c_uint32), ("gene_idx", C.c_uint32)]
+
+
+class ReadScore(C.Structure):
+    """shk_read_score: a read is reported iff n_best > 0 and cov >= c * len (IEEE double) and (not -s or n_best == 1)."""
+    _fields_ = [("len", C.c_uint32), ("cov", C.c_uint32), ("hits", C.c_uint32), ("n_best", C.c_uint32)]
 
 
 class ChunkResult(C.Structure):
@@ -113,6 +118,7 @@ def load():
     L.shk_reads_submit_packed.argtypes = [vp, C.c_uint32, vp, vp, vp, C.c_uint32]
     L.shk_reads_upload_packed.argtypes = [vp, C.c_uint32, vp, vp, vp, C.c_uint32]
     L.shk_result_expand.argtypes = [C.POINTER(ChunkResult), vp, vp]
+    L.shk_reads_scores.argtypes = [vp, C.c_uint32, C.POINTER(C.POINTER(ReadScore)), C.POINTER(C.c_uint32)]
     L.shk_reads_upload.argtypes = [vp, C.c_uint32, vp, vp, vp, C.c_uint32]
     L.shk_reads_analyze_resident.argtypes = [vp, C.c_uint32]
     L.shk_device_timer_start.argtypes = [vp]

@@ -128,13 +128,16 @@ struct Chunk {
     const uint16_t *gene16 = nullptr;
     const AssocPair *multi = nullptr;
     size_t n_multi = 0;
+    const uint32_t *scores = nullptr;  // with a scores output: per read {len, cov, hits, n_best} (shk_read_score)
     std::vector<uint16_t> gene16_v;
     std::vector<AssocPair> multi_v;
+    std::vector<uint32_t> scores_v;
     void results_from_vectors()
     {
         gene16 = gene16_v.data();
         multi = multi_v.data();
         n_multi = multi_v.size();
+        scores = scores_v.empty() ? nullptr : scores_v.data();
     }
     int slot = -1;  // shared slot this chunk's buffers live in (two-process CLI)
     uint32_t n = 0;
@@ -150,7 +153,8 @@ struct Chunk {
         keep.clear();
         gene16_v.clear();
         multi_v.clear();
-        gene16 = nullptr, multi = nullptr, n_multi = 0;
+        scores_v.clear();
+        gene16 = nullptr, multi = nullptr, n_multi = 0, scores = nullptr;
         bulk = false;
         n = 0;
         bytes = 0;
@@ -562,13 +566,16 @@ private:
     size_t cap_, len_ = 0;
 };
 
-// ReadOutput::operator() (ReadOutput.hpp:37-50) for one chunk's results in the compact form.
+// ReadOutput::operator() (ReadOutput.hpp:37-50) for one chunk's results in the compact form.  An optional fourth
+// output (fd_scores >= 0, the chunks carry score records) gets one line per reported read, in the order of the ssv:
+// `<name> <len> <cov> <hits> <n_best>`, name = the ssv's first field (shk_read_score, include/shark_b200.h).
 template <class Alloc>
 class Writer {
 public:
-    Writer(int fd_ssv, int fd_out1, int fd_out2, const std::vector<std::string> &legend, bool paired)
-        : legend_(legend), paired_(paired), ssv_(fd_ssv), out1_(fd_out1), out2_(fd_out2), has1_(fd_out1 >= 0),
-          has2_(fd_out2 >= 0 && paired)
+    static constexpr int kOuts = 4;  // ssv, FASTQ 1, FASTQ 2, scores
+    Writer(int fd_ssv, int fd_out1, int fd_out2, const std::vector<std::string> &legend, bool paired, int fd_scores = -1)
+        : legend_(legend), paired_(paired), ssv_(fd_ssv), out1_(fd_out1), out2_(fd_out2), scores_(fd_scores), has1_(fd_out1 >= 0),
+          has2_(fd_out2 >= 0 && paired), has3_(fd_scores >= 0)
     {
         for (const std::string &g : legend_) legend_len_.push_back((uint32_t)strlen(g.c_str()));
         // Files on tmpfs are written through shared mappings: the threads of the pool fault pages in
@@ -577,8 +584,8 @@ public:
         // 3-4 GB/s there; profiles/iobench_r2.txt), so everything else is formatted into a private buffer and
         // written in order.  SHK_OUT=map / write forces either.
         const char *mode = getenv("SHK_OUT");
-        const int fds[3] = {fd_ssv, has1_ ? fd_out1 : -1, has2_ ? fd_out2 : -1};
-        for (int f = 0; f < 3; ++f) {
+        const int fds[kOuts] = {fd_ssv, has1_ ? fd_out1 : -1, has2_ ? fd_out2 : -1, fd_scores};
+        for (int f = 0; f < kOuts; ++f) {
             struct stat st;
             struct statfs sf;
             const bool can = fds[f] >= 0 && fstat(fds[f], &st) == 0 && S_ISREG(st.st_mode) && lseek(fds[f], 0, SEEK_CUR) >= 0 &&
@@ -601,7 +608,7 @@ public:
     // per page: it allocates the page and can never change what the writer has already stored there.  The file is
     // cut to its real length at the end (flush()).  Only for mapped outputs, and only if the file system has
     // room for twice the bound.
-    void start_prefault(const uint64_t expect[3], int n_threads)
+    void start_prefault(const uint64_t expect[3], int n_threads)  // (ssv and FASTQ outputs)
     {
         OutBuf *outs[3] = {&ssv_, &out1_, &out2_};
         for (int f = 0; f < 3; ++f) {
@@ -637,8 +644,8 @@ public:
     {
         stop_prefault();
         stop_async();
-        OutBuf *outs[3] = {&ssv_, &out1_, &out2_};
-        for (int f = 0; f < 3; ++f) {
+        OutBuf *outs[kOuts] = {&ssv_, &out1_, &out2_, &scores_};
+        for (int f = 0; f < kOuts; ++f) {
             outs[f]->flush();
             if (win_[f].base) {  // the file was grown ahead of the data: cut it to what was written
                 if (ftruncate(outs[f]->fd(), win_[f].pos) != 0) {
@@ -659,22 +666,22 @@ public:
         const size_t n_ranges = std::min<size_t>((size_t)WorkPool::instance().size() * 4, ((size_t)ch.n + 8191) / 8192);
         const size_t per = ((size_t)ch.n + n_ranges - 1) / n_ranges;
         const double t_f = stage_now();
-        std::vector<size_t> at[3];
+        std::vector<size_t> at[kOuts];
         for (auto &v : at) v.assign(n_ranges + 1, 0);
         WorkPool::instance().run(n_ranges, [&](size_t t) {
             const uint32_t a = (uint32_t)(t * per), b = (uint32_t)std::min<size_t>(ch.n, (t + 1) * per);
-            CountSink c[3];
-            format(ch, a, b, c[0], c[1], c[2]);
-            for (int f = 0; f < 3; ++f) at[f][t + 1] = c[f].n;
+            CountSink c[kOuts];
+            format(ch, a, b, c[0], c[1], c[2], c[3]);
+            for (int f = 0; f < kOuts; ++f) at[f][t + 1] = c[f].n;
         });
         for (auto &v : at)
             for (size_t t = 0; t < n_ranges; ++t) v[t + 1] += v[t];
-        OutBuf *outs[3] = {&ssv_, &out1_, &out2_};
-        char *dst[3] = {nullptr, nullptr, nullptr};  // where byte 0 of this chunk's share of output f goes
-        bool mapped[3] = {false, false, false};
-        for (int f = 0; f < 3; ++f) {
+        OutBuf *outs[kOuts] = {&ssv_, &out1_, &out2_, &scores_};
+        char *dst[kOuts] = {nullptr, nullptr, nullptr, nullptr};  // where byte 0 of this chunk's share of output f goes
+        bool mapped[kOuts] = {false, false, false, false};
+        for (int f = 0; f < kOuts; ++f) {
             const size_t total = at[f][n_ranges];
-            if (!total || (f == 1 && !has1_) || (f == 2 && !has2_)) continue;
+            if (!total || (f == 1 && !has1_) || (f == 2 && !has2_) || (f == 3 && !has3_)) continue;
             if (mappable_[f] && (total >= (1u << 16) || win_[f].base)) dst[f] = window(f, total);
             mapped[f] = dst[f] != nullptr;
             if (!dst[f]) {
@@ -689,22 +696,22 @@ public:
         }
         WorkPool::instance().run(n_ranges, [&](size_t t) {
             const uint32_t a = (uint32_t)(t * per), b = (uint32_t)std::min<size_t>(ch.n, (t + 1) * per);
-            WriteSink w[3];
-            for (int f = 0; f < 3; ++f) w[f].p = dst[f] ? dst[f] + at[f][t] : nullptr;
+            WriteSink w[kOuts];
+            for (int f = 0; f < kOuts; ++f) w[f].p = dst[f] ? dst[f] + at[f][t] : nullptr;
 #ifdef MADV_POPULATE_WRITE
             if (populate_)  // allocate this range's pages of the file in one call instead of one fault per page
-                for (int f = 0; f < 3; ++f)
+                for (int f = 0; f < kOuts; ++f)
                     if (mapped[f] && at[f][t + 1] > at[f][t]) {
                         const uintptr_t pg = (uintptr_t)sysconf(_SC_PAGESIZE);
                         const uintptr_t lo = (uintptr_t)(dst[f] + at[f][t]) / pg * pg, hi = (uintptr_t)(dst[f] + at[f][t + 1]);
                         madvise((void *)lo, hi - lo, MADV_POPULATE_WRITE);
                     }
 #endif
-            format(ch, a, b, w[0], w[1], w[2]);
+            format(ch, a, b, w[0], w[1], w[2], w[3]);
         });
         const double t_o = stage_now();
         stage_times().format += t_o - t_f;
-        for (int f = 0; f < 3; ++f) {
+        for (int f = 0; f < kOuts; ++f) {
             const size_t total = at[f][n_ranges];
             if (!dst[f] || !total) continue;
             if (mapped[f]) {
@@ -769,7 +776,18 @@ private:
         return it == ch.batch_start.begin() ? -1 : (int64_t) * (it - 1);
     }
     template <class Sink>
-    void format(const Chunk<Alloc> &ch, uint32_t a, uint32_t b, Sink &ssv, Sink &o1, Sink &o2) const
+    static void put_u32(Sink &o, uint32_t v)
+    {
+        char d[10];
+        int n = 0;
+        do {
+            d[9 - n++] = (char)('0' + v % 10u);
+            v /= 10u;
+        } while (v);
+        o.put(d + 10 - n, (size_t)n);
+    }
+    template <class Sink>
+    void format(const Chunk<Alloc> &ch, uint32_t a, uint32_t b, Sink &ssv, Sink &o1, Sink &o2, Sink &sc) const
     {
         // ReadOutput's previd (ReadOutput.hpp:41,44-48) entering this range: the name of the previous kept read of
         // the same batch - earlier in this chunk, or carried over from the previous chunk
@@ -809,6 +827,15 @@ private:
             } else {
                 for (; m_it != m_end && m_it->read_idx == r; ++m_it) line(m_it->gene_idx);
             }
+            if (has3_ && ch.scores) {
+                const uint32_t *s = ch.scores + 4 * (size_t)r;
+                sc.put(f.name1, f.nlen1);
+                for (int i = 0; i < 4; ++i) {
+                    sc.putc(' ');
+                    put_u32(sc, s[i]);
+                }
+                sc.putc('\n');
+            }
             // FASTQ once per read unless its name equals the previous printed id (ReadOutput.hpp:44-48)
             const bool same = prevlen == f.nlen1 && memcmp(previd, f.name1, prevlen) == 0;
             if (!same) {
@@ -847,8 +874,8 @@ private:
     const std::vector<std::string> &legend_;
     std::vector<uint32_t> legend_len_;
     bool paired_;
-    OutBuf ssv_, out1_, out2_;
-    bool has1_, has2_;
+    OutBuf ssv_, out1_, out2_, scores_;
+    bool has1_, has2_, has3_;
     // Output through mappings: the file is grown a window (1 GiB) at a time and the window mapped once; chunks
     // are formatted into it back to back.  -> address of the next `total` bytes of output f (nullptr: cannot map).
     struct Window {
@@ -866,7 +893,7 @@ private:
     std::atomic<bool> pre_stop_{false};
     char *window(int f, size_t total)
     {
-        OutBuf *outs[3] = {&ssv_, &out1_, &out2_};
+        OutBuf *outs[kOuts] = {&ssv_, &out1_, &out2_, &scores_};
         Window &w = win_[f];
         const int fd = outs[f]->fd();
         if (!w.base) {
@@ -889,19 +916,19 @@ private:
     }
     void abort_windows(int f)  // mapping failed mid-way: continue with write(2) at the current position
     {
-        OutBuf *outs[3] = {&ssv_, &out1_, &out2_};
+        OutBuf *outs[kOuts] = {&ssv_, &out1_, &out2_, &scores_};
         if (ftruncate(outs[f]->fd(), win_[f].pos) != 0) {
         }
         lseek(outs[f]->fd(), win_[f].pos, SEEK_SET);
         win_[f] = Window{};
         mappable_[f] = false;
     }
-    Window win_[3];
-    bool mappable_[3] = {false, false, false};  // a regular file opened read-write (a shared mapping needs both)
+    Window win_[kOuts];
+    bool mappable_[kOuts] = {false, false, false, false};  // a regular file opened read-write (a shared mapping needs both)
     bool populate_ = false;
-    std::vector<char> priv_[3][2];
-    int priv_turn_[3] = {0, 0, 0};
-    uint64_t priv_job_[3][2] = {{0, 0}, {0, 0}, {0, 0}};
+    std::vector<char> priv_[kOuts][2];
+    int priv_turn_[kOuts] = {0, 0, 0, 0};
+    uint64_t priv_job_[kOuts][2] = {{0, 0}, {0, 0}, {0, 0}, {0, 0}};
     // background write(2) of private buffers, in submission order
     struct AsyncJob {
         OutBuf *ob;

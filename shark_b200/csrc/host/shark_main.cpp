@@ -8,7 +8,9 @@
 // (with --gpus N: every GPU indexes one gene shard, filters OR-merged over NVLink, instead of build +
 // replicate), --save-index FILE / --load-index FILE (the reference rebuilds its index on every run;
 // the gene names still come from -r), --wide-ids (32-bit gene ids: references of more than 65536 records, which
-// the reference's 16-bit ids cannot index - small_vector.hpp:46; without the flag such inputs end with an error).
+// the reference's 16-bit ids cannot index - small_vector.hpp:46; without the flag such inputs end with an error),
+// --scores FILE (one line `<name> <len> <cov> <hits> <n_best>` per reported read, in the order of the ssv: the numbers
+// behind each answer, from which any -c / -s can be applied afterwards - shk_read_score, include/shark_b200.h).
 //
 // Pipeline (pipeline.hpp, fastpipe.hpp, ingest.hpp): plain input files are memory-mapped and scanned by
 // the host pool in parallel (compressed ones by a streaming scanner per file); a batcher thread turns runs
@@ -83,6 +85,7 @@ struct Options {
     bool sharded_build = false;     // extension
     bool wide_ids = false;          // extension: more than 65536 reference records (SHK_F_WIDE_IDS)
     std::string save_index, load_index;  // extensions
+    std::string scores_path;        // extension: per-read score records (SHK_F_SCORES)
 };
 
 [[noreturn]] void usage_error(const char *msg, bool with_usage)
@@ -154,6 +157,7 @@ const OptionRow kOptions[] = {
     {1003, "save-index", true, [](Options &o, std::istringstream &a) { a >> o.save_index; }},
     {1004, "load-index", true, [](Options &o, std::istringstream &a) { a >> o.load_index; }},
     {1005, "wide-ids", false, [](Options &o, std::istringstream &) { o.wide_ids = true; }},
+    {1006, "scores", true, [](Options &o, std::istringstream &a) { a >> o.scores_path; }},
 };
 
 Options parse_arguments(int argc, char **argv)
@@ -287,7 +291,7 @@ private:
 //     finishes on its own ("detached tear-down").
 // The two share one anonymous mapping created before the fork: per chunk buffer a slot with the packed chunk
 // (offsets, code words, validity words; host -> device) and the compact results (one 16-bit word per read + the
-// list for ties; device -> host).  Two pipes carry the small messages.  SHK_ONE_PROCESS=1 runs the device side as
+// list for ties, and with --scores the score records, 16 bytes per read; device -> host).  Two pipes carry the small messages.  SHK_ONE_PROCESS=1 runs the device side as
 // a thread of the host process instead (same protocol; for debuggers and sanitizers).
 // ---------------------------------------------------------------------------------------------------------
 struct SlotView {
@@ -296,13 +300,14 @@ struct SlotView {
     uint32_t *valid;
     uint16_t *gene16;
     shkhost::AssocPair *multi;
+    uint32_t *scores;  // nullptr without --scores
 };
 struct SharedLayout {
     char *base = nullptr;
     size_t n_slots = 0, slot_bytes = 0;
-    size_t off_bytes = 0, codes_bytes = 0, valid_bytes = 0, gene_bytes = 0, multi_cap = 0;
+    size_t off_bytes = 0, codes_bytes = 0, valid_bytes = 0, gene_bytes = 0, multi_cap = 0, scores_bytes = 0;
     static size_t round(size_t n) { return (n + 4095) / 4096 * 4096; }
-    void plan(size_t slots, size_t max_reads, uint64_t max_bytes)
+    void plan(size_t slots, size_t max_reads, uint64_t max_bytes, bool scores)
     {
         n_slots = slots;
         const size_t groups = (size_t)((max_bytes + 31) / 32) + 2;
@@ -311,7 +316,8 @@ struct SharedLayout {
         valid_bytes = round(groups * 4 + 64);
         gene_bytes = round((max_reads + 64) * 2);
         multi_cap = max_reads;  // entries; a chunk with more ties than reads sends the rest through the pipe
-        slot_bytes = off_bytes + codes_bytes + valid_bytes + gene_bytes + round(multi_cap * sizeof(shkhost::AssocPair));
+        scores_bytes = scores ? round(max_reads * sizeof(shk_read_score)) : 0;
+        slot_bytes = off_bytes + codes_bytes + valid_bytes + gene_bytes + round(multi_cap * sizeof(shkhost::AssocPair)) + scores_bytes;
     }
     bool map()
     {
@@ -329,6 +335,7 @@ struct SharedLayout {
         v.valid = (uint32_t *)(p + off_bytes + codes_bytes);
         v.gene16 = (uint16_t *)(p + off_bytes + codes_bytes + valid_bytes);
         v.multi = (shkhost::AssocPair *)(p + off_bytes + codes_bytes + valid_bytes + gene_bytes);
+        v.scores = scores_bytes ? (uint32_t *)(p + slot_bytes - scores_bytes) : nullptr;
         return v;
     }
 };
@@ -415,7 +422,7 @@ void device_main(const Options &opt, const SharedLayout &shm, unsigned chunk_rea
         p.n_slots = 2;
         p.max_reads_per_chunk = chunk_reads;
         p.max_bytes_per_chunk = max_chunk_bytes;
-        p.flags = SHK_F_COMPACT_RESULTS | (opt.wide_ids ? SHK_F_WIDE_IDS : 0u);
+        p.flags = SHK_F_COMPACT_RESULTS | (opt.wide_ids ? SHK_F_WIDE_IDS : 0u) | (opt.scores_path.empty() ? 0u : SHK_F_SCORES);
         if (shk_create(&p, &ctxs[g]) != SHK_OK) die(std::string("shk_create: ") + shk_last_error(nullptr));
     }
     tstamp("contexts created");
@@ -468,6 +475,12 @@ void device_main(const Options &opt, const SharedLayout &shm, unsigned chunk_rea
         memcpy(v.gene16, res.gene16, (size_t)res.n_reads * 2);
         const uint64_t in_slot = std::min<uint64_t>(res.n_multi, shm.multi_cap);
         if (in_slot) memcpy(v.multi, res.multi, in_slot * sizeof(shk_assoc));
+        if (v.scores) {
+            const shk_read_score *sc = nullptr;
+            uint32_t n_sc = 0;
+            SHK_TRY(ctxs[f.gpu], shk_reads_scores(ctxs[f.gpu], f.slot, &sc, &n_sc));
+            memcpy(v.scores, sc, (size_t)n_sc * sizeof(shk_read_score));
+        }
         Msg m;
         m.kind = kMsgResult;
         m.slot = f.shm_slot;
@@ -543,7 +556,7 @@ int main(int argc, char *argv[])
         close(fd);
     }
     SharedLayout shm;
-    shm.plan(n_bufs, chunk_reads, max_chunk_bytes);
+    shm.plan(n_bufs, chunk_reads, max_chunk_bytes, !opt.scores_path.empty());
     if (!shm.map()) die("cannot map the chunk buffers");
     int h2d[2], d2h[2];
     if (pipe(h2d) != 0 || pipe(d2h) != 0) die("cannot create pipes");
@@ -647,7 +660,9 @@ int main(int argc, char *argv[])
     }
     const int fd1 = opt.out1_path.empty() ? -1 : open(opt.out1_path.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0666);
     const int fd2 = (!opt.paired || opt.out2_path.empty()) ? -1 : open(opt.out2_path.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0666);
-    Writer writer(STDOUT_FILENO, fd1, fd2, legend_ID, opt.paired);
+    const int fd_scores = opt.scores_path.empty() ? -1 : open(opt.scores_path.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0666);
+    if (!opt.scores_path.empty() && fd_scores < 0) die("cannot create " + opt.scores_path);
+    Writer writer(STDOUT_FILENO, fd1, fd2, legend_ID, opt.paired, fd_scores);
     if (!(getenv("SHK_PREFAULT") && atoi(getenv("SHK_PREFAULT")) == 0)) {
         // the filtered FASTQ of a FASTQ sample is never longer than the sample (pipeline.hpp, Writer::start_prefault)
         auto plain_size = [](const std::string &path) -> uint64_t {
@@ -690,6 +705,7 @@ int main(int argc, char *argv[])
         Chunk *ch = pool[m.slot].get();
         const SlotView v = shm.slot(m.slot);
         ch->gene16 = v.gene16;
+        ch->scores = v.scores;
         if (m.tail) {  // more ties than the slot holds: the whole list, slot part + pipe part, in the chunk's own vector
             ch->multi_v.resize((size_t)m.n_multi);
             memcpy(ch->multi_v.data(), v.multi, (size_t)(m.n_multi - m.tail) * sizeof(shkhost::AssocPair));
@@ -713,6 +729,7 @@ int main(int argc, char *argv[])
     writer_thread.join();
     if (fd1 >= 0) close(fd1);
     if (fd2 >= 0) close(fd2);
+    if (fd_scores >= 0) close(fd_scores);
     tstamp("output written");
     if (g_timing) {
         const shkhost::StageTimes &st = shkhost::stage_times();

@@ -312,7 +312,8 @@ __device__ SHK_BULK_SERVE_ATTR void serve_queue(const ReadKernelArgs &a, BulkWar
     }
 }
 
-template <int MOD>
+// SCORES: also store each settled read's score record (SHK_F_SCORES); the instantiations without it are the default path.
+template <int MOD, bool SCORES>
 __global__ void __launch_bounds__(kBulkThreads, SHK_BULK_MIN_BLOCKS)
 analyze_bulk_kernel(const ReadKernelArgs a)
 {
@@ -627,7 +628,9 @@ analyze_bulk_kernel(const ReadKernelArgs a)
             sh.n_probes[lane] = 0, sh.n_hits[lane] = 0;  // counted by the kernel that classifies the read
             a.slow_list[atomicAdd(&a.counters->n_slow, 1u)] = r;
         } else {
-            finish_read(a, tab.full(cold), sh.n_len[lane], count, payload);
+            uint4 score;
+            finish_read(a, tab.full(cold), sh.n_len[lane], count, payload, score);
+            if (SCORES) a.scores[r] = score;  // (a slow read's record comes from the kernel that settles it)
         }
         a.rec[r] = make_uint2(count, payload);
     }
@@ -656,13 +659,16 @@ bool bulk_enabled()
     return e[0] != '0';
 }
 
+template <bool SCORES>
 void launch_bulk_kernel(const ReadKernelArgs &a, cudaStream_t st, unsigned blocks)
 {
     switch (a.geom.mod_kind) {
-    case MOD_POW2: analyze_bulk_kernel<MOD_POW2><<<blocks, kBulkThreads, 0, st>>>(a); break;
-    case MOD_B33: analyze_bulk_kernel<MOD_B33><<<blocks, kBulkThreads, 0, st>>>(a); break;
-    default: analyze_bulk_kernel<MOD_GENERIC><<<blocks, kBulkThreads, 0, st>>>(a); break;
+    case MOD_POW2: analyze_bulk_kernel<MOD_POW2, SCORES><<<blocks, kBulkThreads, 0, st>>>(a); break;
+    case MOD_B33: analyze_bulk_kernel<MOD_B33, SCORES><<<blocks, kBulkThreads, 0, st>>>(a); break;
+    default: analyze_bulk_kernel<MOD_GENERIC, SCORES><<<blocks, kBulkThreads, 0, st>>>(a); break;
     }
 }
+template void launch_bulk_kernel<false>(const ReadKernelArgs &, cudaStream_t, unsigned);
+template void launch_bulk_kernel<true>(const ReadKernelArgs &, cudaStream_t, unsigned);
 
 }  // namespace shk

@@ -61,6 +61,8 @@ static void free_slot(Slot &s)
     free(s.h_keep);
     cudaFreeHost(s.h_pack);
     cudaFree(s.d_pack);
+    cudaFree(s.d_scores);
+    cudaFreeHost(s.h_scores);
     if (s.ev_start) cudaEventDestroy(s.ev_start);
     if (s.ev_k0) cudaEventDestroy(s.ev_k0);
     if (s.ev_ka) cudaEventDestroy(s.ev_ka);
@@ -199,6 +201,10 @@ static int alloc_slot(shk_ctx *ctx, Slot &s)
     s.h_multi_cap = s.multi_cap;
     SHK_CUDA(ctx, pinned_alloc((void **)&s.h_multi, s.h_multi_cap * sizeof(shk_assoc)));
     SHK_CUDA(ctx, pinned_alloc((void **)&s.h_gene16, (R + 64) * 2));
+    if (ctx->scores) {
+        SHK_CUDA(ctx, cudaMalloc((void **)&s.d_scores, R * sizeof(uint4)));
+        SHK_CUDA(ctx, pinned_alloc((void **)&s.h_scores, R * sizeof(shk_read_score)));
+    }
     // packed reads: + 2 groups so that the kernels' prefetch of the following group stays inside
     s.pack_groups_cap = (B + 31) / 32 + 2;
     SHK_CUDA(ctx, cudaMalloc((void **)&s.d_pack, s.pack_groups_cap * 12));
@@ -260,6 +266,7 @@ static ReadKernelArgs make_args(shk_ctx *ctx, Slot &s)
     a.tile_base = s.d_tile_base;
     a.gene16 = s.d_gene16;
     a.multi = s.d_multi;
+    a.scores = s.d_scores;
     return a;
 }
 
@@ -289,6 +296,7 @@ static int ensure_slow_table(shk_ctx *ctx)
 
 static int enqueue_chunk_kernels(shk_ctx *ctx, Slot &s)
 {
+    s.collected = false;
     SHK_CUDA(ctx, cudaMemsetAsync(s.d_counters, 0, sizeof(ChunkCounters), s.stream));
     ReadKernelArgs a = make_args(ctx, s);
     s.launches += (uint32_t)launch_read_kernels(ctx, a, s.multi_cap, s.stream, s.ev_k0, s.ev_ka, s.ev_k1);
@@ -306,6 +314,11 @@ static int enqueue_chunk_kernels(shk_ctx *ctx, Slot &s)
     if (pre) SHK_CUDA(ctx, cudaMemcpyAsync(s.h_multi, s.d_multi, pre * sizeof(shk_assoc), cudaMemcpyDeviceToHost, s.stream));
     s.pre_multi = pre;
     ctx->d2h_bytes += pre * sizeof(shk_assoc) + (uint64_t)s.n_reads * 2 + sizeof(ChunkCounters);
+    if (s.h_scores && s.n_reads) {
+        SHK_CUDA(ctx, cudaMemcpyAsync(s.h_scores, s.d_scores, (size_t)s.n_reads * sizeof(shk_read_score), cudaMemcpyDeviceToHost,
+                                      s.stream));
+        ctx->d2h_bytes += (uint64_t)s.n_reads * sizeof(shk_read_score);
+    }
     SHK_CUDA(ctx, cudaEventRecord(s.ev_done, s.stream));
     return SHK_OK;
 }
@@ -394,6 +407,7 @@ static int enqueue_upload(shk_ctx *ctx, Slot &s, const uint8_t *seq, const uint8
                           uint32_t n_reads, bool allow_pack)
 {
     s.n_reads = n_reads;
+    s.collected = false;
     s.n_bytes = n_reads ? off[n_reads] : 0;
     s.has_qual = (ctx->params.min_quality & 0xFF) != 0;
     s.launches = 0;
@@ -447,6 +461,7 @@ static int enqueue_upload_packed(shk_ctx *ctx, Slot &s, const uint64_t *codes, c
                                  uint32_t n_reads)
 {
     s.n_reads = n_reads;
+    s.collected = false;
     s.n_bytes = n_reads ? off[n_reads] : 0;
     s.has_qual = false;
     s.launches = 0;
@@ -463,6 +478,7 @@ static int enqueue_upload_packed(shk_ctx *ctx, Slot &s, const uint64_t *codes, c
 
 using namespace shk;
 
+static_assert(sizeof(shk_read_score) == sizeof(uint4), "the kernels store a score record as one uint4");
 static_assert(sizeof(shk_index_info) == 96 && sizeof(shk_shard_mem) == 240 && sizeof(shk_chunk_result) == 112, "layouts mirrored in shark_b200/capi.py");
 
 extern "C" {
@@ -480,7 +496,7 @@ int shk_create(const shk_params *p, shk_ctx **out)
     if (p->bf_bits < 64) return fail(nullptr, SHK_E_ARG, "bf_bits must be >= 64");
     if ((p->flags & SHK_F_EXTEND_ON) && (p->flags & SHK_F_EXTEND_OFF))
         return fail(nullptr, SHK_E_ARG, "SHK_F_EXTEND_ON and SHK_F_EXTEND_OFF are exclusive");
-    if (p->flags & ~(SHK_F_EXTEND_ON | SHK_F_EXTEND_OFF | SHK_F_HOST_PACK | SHK_F_COMPACT_RESULTS | SHK_F_WIDE_IDS))
+    if (p->flags & ~(SHK_F_EXTEND_ON | SHK_F_EXTEND_OFF | SHK_F_HOST_PACK | SHK_F_COMPACT_RESULTS | SHK_F_WIDE_IDS | SHK_F_SCORES))
         return fail(nullptr, SHK_E_ARG, "unknown flag bits");
     if ((p->flags & SHK_F_WIDE_IDS) && (p->flags & SHK_F_EXTEND_ON))
         return fail(nullptr, SHK_E_ARG, "SHK_F_WIDE_IDS has no extension structures (SHK_F_EXTEND_ON)");
@@ -504,6 +520,7 @@ int shk_create(const shk_params *p, shk_ctx **out)
     ctx->host_pack = (p->flags & SHK_F_HOST_PACK) != 0;
     ctx->compact_results = (p->flags & SHK_F_COMPACT_RESULTS) != 0;
     ctx->wide_ids = (p->flags & SHK_F_WIDE_IDS) != 0;
+    ctx->scores = (p->flags & SHK_F_SCORES) != 0;
     if (const char *ev = getenv("SHK_HOST_PACK")) ctx->host_pack = atoi(ev) != 0;  // tuning override
     int rc = SHK_OK;
     auto bail = [&](int code) {
@@ -1230,6 +1247,7 @@ int shk_reads_collect(shk_ctx *ctx, uint32_t slot, shk_chunk_result *out)
     out->n_extended = c.n_extended;
     out->n_table_loads = c.n_table_loads;
     s.pending = false;
+    s.collected = true;
     if (!ctx->compact_results) {
         // the classic form of the ABI: association list + keep flags, expanded here on the calling thread
         if (c.n_assoc > s.h_assoc_cap || !s.h_assoc) {
@@ -1247,6 +1265,17 @@ int shk_reads_collect(shk_ctx *ctx, uint32_t slot, shk_chunk_result *out)
         out->assoc = s.h_assoc;
         out->keep = s.h_keep;
     }
+    return SHK_OK;
+}
+
+int shk_reads_scores(shk_ctx *ctx, uint32_t slot, const shk_read_score **scores, uint32_t *n_reads)
+{
+    if (!ctx || slot >= ctx->n_slots || !scores || !n_reads) return fail(ctx, SHK_E_ARG, "bad argument");
+    if (!ctx->scores) return fail(ctx, SHK_E_STATE, "the context was created without SHK_F_SCORES");
+    const Slot &s = ctx->slots[slot];
+    if (!s.collected) return fail(ctx, SHK_E_STATE, "slot %u has no collected chunk", slot);
+    *scores = s.h_scores;
+    *n_reads = s.n_reads;
     return SHK_OK;
 }
 

@@ -112,6 +112,9 @@ struct ReadKernelArgs {
     uint32_t *tile_base;
     uint16_t *gene16;        // per read: gene index, SHK_GENE_NONE or SHK_GENE_MULTI
     shk_assoc *multi;        // associations of the SHK_GENE_MULTI reads, ordered by read then gene
+    // SHK_F_SCORES: per read {len, cov, hits, n_best} (shk_read_score), written by the kernel that settles the read;
+    // nullptr without the flag (the kernels without scores never touch it)
+    uint4 *scores;
 };
 
 constexpr uint32_t kReadsPerTile = 128;  // one CTA of the fast kernel: 128 threads = 128 reads
@@ -151,11 +154,15 @@ struct Slot {
     uint64_t *h_pack = nullptr, *d_pack = nullptr;
     uint64_t pack_groups_cap = 0;
     uint32_t pack_first = 0xFFFFFFFFu, pack_base = 0;  // this chunk: reads >= pack_first are packed
+    // SHK_F_SCORES only: one record per read, read back with the other results
+    uint4 *d_scores = nullptr;
+    shk_read_score *h_scores = nullptr;
     // state
     uint32_t n_reads = 0;
     uint64_t n_bytes = 0;
     bool has_qual = false;
     bool pending = false;
+    bool collected = false;  // the results of the slot's last chunk are on the host (shk_reads_scores)
     uint32_t launches = 0;
 };
 
@@ -214,6 +221,7 @@ struct shk_ctx {
     std::atomic<double> multi_per_read{-1.0};  // last chunk's multi entries per read: sizes the early read-back
     bool compact_results = false;          // SHK_F_COMPACT_RESULTS
     bool wide_ids = false;                 // SHK_F_WIDE_IDS
+    bool scores = false;                   // SHK_F_SCORES
     shk::PackControl pack;                 // split upload: feedback state of the packed share
     char err[512] = {0};
 };
@@ -264,6 +272,7 @@ int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t assoc_ca
 int launch_scatter(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t assoc_cap, cudaStream_t st);
 // shk_bulk.cu: the bulk classification kernel for packed reads over the extension structures
 bool bulk_enabled();
+template <bool SCORES>
 void launch_bulk_kernel(const ReadKernelArgs &a, cudaStream_t st, unsigned blocks);
 int fetch_cache_policies(shk_ctx *ctx);
 

@@ -224,7 +224,9 @@ __device__ __forceinline__ void codes4(uint32_t w, uint32_t &code4, uint32_t &x)
 // PACKED: the read comes from the packed stream (64-bit code words + 32-bit validity words per 32 bases,
 // shk_hostpack.h) instead of text: no text or quality loads, no byte-parallel decode; the -q masking rule is
 // already in the validity bits.  Everything from the rolling k-mers on is the same code.
-template <bool HAS_QUAL, int MOD, bool EXT, bool PACKED>
+//
+// SCORES: also store each settled read's score record (SHK_F_SCORES); the instantiations without it are the default path.
+template <bool HAS_QUAL, int MOD, bool EXT, bool PACKED, bool SCORES>
 __global__ void __launch_bounds__(kFastThreads, EXT ? SHK_EXT_MIN_BLOCKS : SHK_FAST_MIN_BLOCKS)
 analyze_reads_kernel(const ReadKernelArgs a)
 {
@@ -246,6 +248,7 @@ analyze_reads_kernel(const ReadKernelArgs a)
     const uint32_t fshift = a.fgeom.shift, fmask = a.fgeom.off_mask;
     const uint32_t mq4b = (0x01010101u * (uint32_t)(a.mq & 0xFF)) ^ kH4;
     uint32_t count = 0, payload = 0, my_probes = 0, my_hits = 0, my_ext = 0, my_loads = 0;
+    uint4 score = make_uint4(0u, 0u, 0u, 0u);
     bool slow = false;
 
     if (r < a.r1) {
@@ -468,7 +471,7 @@ analyze_reads_kernel(const ReadKernelArgs a)
             if (tab.overflow) {
                 slow = true;
             } else {
-                finish_read(a, tab, len, count, payload);
+                finish_read(a, tab, len, count, payload, score);
             }
         }
         if (slow) {
@@ -478,6 +481,7 @@ analyze_reads_kernel(const ReadKernelArgs a)
             a.slow_list[atomicAdd(&a.counters->n_slow, 1u)] = r;
         }
         a.rec[r] = make_uint2(count, payload);
+        if (SCORES && !slow) a.scores[r] = score;  // (a slow read's record comes from the kernel that settles it)
     }
     // every warp retires on its own (tile_sums is zeroed before the launch): no warp of a CTA
     // waits at a barrier for its slowest sibling
@@ -512,7 +516,7 @@ analyze_reads_kernel(const ReadKernelArgs a)
 // ---------------------------------------------------------------------------------------------
 constexpr uint32_t kMidSlots = 128, kMidMaxGenes = 95, kMidWarps = 4;
 
-template <bool HAS_QUAL, int MOD, bool WIDE>
+template <bool HAS_QUAL, int MOD, bool WIDE, bool SCORES>
 __global__ void __launch_bounds__(kMidWarps * 32) analyze_mid_kernel(const ReadKernelArgs a)
 {
     __shared__ uint4 tables[kMidWarps][kMidSlots];  // {gene (0xFFFFFFFF = free), cov, hits, last}
@@ -623,6 +627,7 @@ __global__ void __launch_bounds__(kMidWarps * 32) analyze_mid_kernel(const ReadK
         }
         count = __reduce_add_sync(kFull, count);
         first_gene = __reduce_min_sync(kFull, first_gene);
+        const uint32_t n_best = count;
         const bool pass = count > 0 && wmaxc > 0 && (double)wmaxc >= __dmul_rn(a.c, (double)len) &&
                           (!a.single || count == 1);
         if (!pass) count = 0;
@@ -646,6 +651,7 @@ __global__ void __launch_bounds__(kMidWarps * 32) analyze_mid_kernel(const ReadK
         }
         if (lane == 0) {
             a.rec[r] = make_uint2(count, payload);
+            if (SCORES) a.scores[r] = make_uint4(len, wmaxc, wmaxh, n_best);
             if (multi_entries(count, payload, a.wide)) atomicAdd(&a.tile_sums[r / kReadsPerTile], count);
             assoc_total += count;
             kept_total += count ? 1u : 0u;
@@ -666,7 +672,7 @@ __global__ void __launch_bounds__(kMidWarps * 32) analyze_mid_kernel(const ReadK
 // updated window by window in read order exactly as ReadAnalyzer.hpp:56-62,79-86 does, the
 // lanes sharing the (distinct) ids of one list.  Stamps make clearing unnecessary.
 // ---------------------------------------------------------------------------------------------
-template <bool HAS_QUAL, int MOD, bool WIDE>
+template <bool HAS_QUAL, int MOD, bool WIDE, bool SCORES>
 __global__ void __launch_bounds__(128) analyze_slow_kernel(const ReadKernelArgs a)
 {
     const int lane = threadIdx.x & 31;
@@ -753,6 +759,7 @@ __global__ void __launch_bounds__(128) analyze_slow_kernel(const ReadKernelArgs 
             if (b && first_gene == 0xFFFFFFFFu) first_gene = g0 + (uint32_t)(__ffs(b) - 1);
             count += __popc(b);
         }
+        const uint32_t n_best = count;
         const bool pass = count > 0 && wmaxc > 0 && (double)wmaxc >= __dmul_rn(a.c, (double)len) &&
                           (!a.single || count == 1);
         if (!pass) count = 0;
@@ -776,6 +783,7 @@ __global__ void __launch_bounds__(128) analyze_slow_kernel(const ReadKernelArgs 
         }
         if (lane == 0) {
             a.rec[r] = make_uint2(count, payload);
+            if (SCORES) a.scores[r] = make_uint4(len, wmaxc, wmaxh, n_best);
             if (multi_entries(count, payload, a.wide)) atomicAdd(&a.tile_sums[r / kReadsPerTile], count);
             assoc_total += count;
             kept_total += count ? 1u : 0u;
@@ -836,7 +844,7 @@ __global__ void __launch_bounds__(256) all_reads_slow_kernel(const ReadKernelArg
     if (r == 0) a.counters->n_slow = a.n_reads;
 }
 
-template <bool HAS_QUAL, int MOD>
+template <bool HAS_QUAL, int MOD, bool SCORES>
 static void launch_typed(const ReadKernelArgs &a0, cudaStream_t st, unsigned tiles, unsigned slow_blocks, cudaEvent_t ev_ka)
 {
     // middle path: a grid-stride loop over the slow list (its length is only known on the device)
@@ -845,8 +853,8 @@ static void launch_typed(const ReadKernelArgs &a0, cudaStream_t st, unsigned til
     if (a.wide) {
         all_reads_slow_kernel<<<(a.n_reads + 255) / 256, 256, 0, st>>>(a);
         if (ev_ka) cudaEventRecord(ev_ka, st);
-        analyze_mid_kernel<HAS_QUAL, MOD, true><<<mid_blocks, kMidWarps * 32, 0, st>>>(a);
-        analyze_slow_kernel<HAS_QUAL, MOD, true><<<slow_blocks, 128, 0, st>>>(a);
+        analyze_mid_kernel<HAS_QUAL, MOD, true, SCORES><<<mid_blocks, kMidWarps * 32, 0, st>>>(a);
+        analyze_slow_kernel<HAS_QUAL, MOD, true, SCORES><<<slow_blocks, 128, 0, st>>>(a);
         return;
     }
     const uint32_t split = std::min(a.pack_first, a.n_reads);
@@ -858,8 +866,8 @@ static void launch_typed(const ReadKernelArgs &a0, cudaStream_t st, unsigned til
         a.r1 = split;
         if (a.front_plain) a.front = a.front_plain;
         const unsigned blocks = (split + kReadsPerTile - 1) / kReadsPerTile;
-        if (ext) analyze_reads_kernel<HAS_QUAL, MOD, true, false><<<blocks, kFastThreads, 0, st>>>(a);
-        else analyze_reads_kernel<HAS_QUAL, MOD, false, false><<<blocks, kFastThreads, 0, st>>>(a);
+        if (ext) analyze_reads_kernel<HAS_QUAL, MOD, true, false, SCORES><<<blocks, kFastThreads, 0, st>>>(a);
+        else analyze_reads_kernel<HAS_QUAL, MOD, false, false, SCORES><<<blocks, kFastThreads, 0, st>>>(a);
         a.front = a0.front;
     }
     if (split < a.n_reads) {  // packed part
@@ -867,17 +875,28 @@ static void launch_typed(const ReadKernelArgs &a0, cudaStream_t st, unsigned til
         a.r1 = a.n_reads;
         const unsigned blocks = (a.n_reads - split + kReadsPerTile - 1) / kReadsPerTile;
         if (a.estream && a.refr && bulk_enabled()) {
-            launch_bulk_kernel(a, st, blocks);
+            launch_bulk_kernel<SCORES>(a, st, blocks);
         } else {
             if (a.front_plain) a.front = a.front_plain;
-            if (ext) analyze_reads_kernel<false, MOD, true, true><<<blocks, kFastThreads, 0, st>>>(a);
-            else analyze_reads_kernel<false, MOD, false, true><<<blocks, kFastThreads, 0, st>>>(a);
+            if (ext) analyze_reads_kernel<false, MOD, true, true, SCORES><<<blocks, kFastThreads, 0, st>>>(a);
+            else analyze_reads_kernel<false, MOD, false, true, SCORES><<<blocks, kFastThreads, 0, st>>>(a);
             a.front = a0.front;
         }
     }
     if (ev_ka) cudaEventRecord(ev_ka, st);
-    analyze_mid_kernel<HAS_QUAL, MOD, false><<<mid_blocks, kMidWarps * 32, 0, st>>>(a);
-    analyze_slow_kernel<HAS_QUAL, MOD, false><<<slow_blocks, 128, 0, st>>>(a);
+    analyze_mid_kernel<HAS_QUAL, MOD, false, SCORES><<<mid_blocks, kMidWarps * 32, 0, st>>>(a);
+    analyze_slow_kernel<HAS_QUAL, MOD, false, SCORES><<<slow_blocks, 128, 0, st>>>(a);
+}
+
+template <bool SCORES>
+static void launch_classify(const ReadKernelArgs &a, cudaStream_t st, unsigned tiles, unsigned slow_blocks, cudaEvent_t ev_ka)
+{
+    const bool q = a.qual != nullptr;
+    switch (a.geom.mod_kind) {
+    case MOD_POW2: q ? launch_typed<true, MOD_POW2, SCORES>(a, st, tiles, slow_blocks, ev_ka) : launch_typed<false, MOD_POW2, SCORES>(a, st, tiles, slow_blocks, ev_ka); break;
+    case MOD_B33: q ? launch_typed<true, MOD_B33, SCORES>(a, st, tiles, slow_blocks, ev_ka) : launch_typed<false, MOD_B33, SCORES>(a, st, tiles, slow_blocks, ev_ka); break;
+    default: q ? launch_typed<true, MOD_GENERIC, SCORES>(a, st, tiles, slow_blocks, ev_ka) : launch_typed<false, MOD_GENERIC, SCORES>(a, st, tiles, slow_blocks, ev_ka); break;
+    }
 }
 
 int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t multi_cap, cudaStream_t st, cudaEvent_t ev_k0,
@@ -888,13 +907,9 @@ int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t multi_ca
     if (a.n_reads > 0) {
         const unsigned tiles = (a.n_reads + kReadsPerTile - 1) / kReadsPerTile;
         const unsigned slow_blocks = (a.n_slow_slabs + 3) / 4;
-        const bool q = a.qual != nullptr;
         cudaMemsetAsync(a.tile_sums, 0, (size_t)tiles * 4, st);  // the classification kernels add to it
-        switch (a.geom.mod_kind) {
-        case MOD_POW2: q ? launch_typed<true, MOD_POW2>(a, st, tiles, slow_blocks, ev_ka) : launch_typed<false, MOD_POW2>(a, st, tiles, slow_blocks, ev_ka); break;
-        case MOD_B33: q ? launch_typed<true, MOD_B33>(a, st, tiles, slow_blocks, ev_ka) : launch_typed<false, MOD_B33>(a, st, tiles, slow_blocks, ev_ka); break;
-        default: q ? launch_typed<true, MOD_GENERIC>(a, st, tiles, slow_blocks, ev_ka) : launch_typed<false, MOD_GENERIC>(a, st, tiles, slow_blocks, ev_ka); break;
-        }
+        if (a.scores) launch_classify<true>(a, st, tiles, slow_blocks, ev_ka);
+        else launch_classify<false>(a, st, tiles, slow_blocks, ev_ka);
         // tile_base <- exclusive scan(tile_sums); the grand total lands in tile_base[tiles]
         cudaMemcpyAsync(a.tile_base, a.tile_sums, (size_t)tiles * 4, cudaMemcpyDeviceToDevice, st);
         scan_tile_sums_kernel<<<1, 1024, 0, st>>>(a.tile_base, tiles, a.tile_base + tiles);

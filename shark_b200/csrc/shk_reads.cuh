@@ -76,9 +76,10 @@ struct Mru4 {
     }
 };
 
-// argmax with ties (ReadAnalyzer.hpp:90-102), threshold and -s (ReadAnalyzer.hpp:104): -> {count, gene | pool offset}
+// argmax with ties (ReadAnalyzer.hpp:90-102), threshold and -s (ReadAnalyzer.hpp:104): -> {count, gene | pool offset},
+// and the read's score record {len, cov, hits, n_best} (SHK_F_SCORES; dead code for the kernels that do not store it)
 __device__ __forceinline__ void finish_read(const ReadKernelArgs &a, const Mru4 &tab, uint32_t len, uint32_t &count,
-                                            uint32_t &payload)
+                                            uint32_t &payload, uint4 &score)
 {
     const uint32_t tg[4] = {tab.g0, tab.g1, tab.g2, tab.g3}, tc[4] = {tab.c0, tab.c1, tab.c2, tab.c3},
                    th[4] = {tab.h0, tab.h1, tab.h2, tab.h3};
@@ -97,6 +98,7 @@ __device__ __forceinline__ void finish_read(const ReadKernelArgs &a, const Mru4 
         wg[i] = is ? tg[i] : 0xFFFFFFFFu;
         count += is ? 1u : 0u;
     }
+    score = make_uint4(len, maxc, maxh, count);
     const bool pass = count > 0 && (double)maxc >= __dmul_rn(a.c, (double)len) && (!a.single || count == 1);
     if (!pass) count = 0;
     if (count == 1) {

@@ -16,17 +16,21 @@ from . import capi
 class Shark:
     def __init__(self, k=17, c=0.6, bf_bits=1 << 33, min_quality=0, single=False, device=0, n_slots=2,
                  max_reads_per_chunk=1 << 20, max_bytes_per_chunk=0, extend=None, host_pack=False, compact=False,
-                 wide_ids=False):
+                 wide_ids=False, scores=False):
         """extend: None = automatic (anchor-and-extend when the front table is DRAM-sized), True /
         False = force it on / off (results are identical; tests run both).  compact: results stay in the
-        compact form (gene16 / multi), shk_reads_collect does no per-read host work."""
+        compact form (gene16 / multi), shk_reads_collect does no per-read host work.  scores: every result also
+        carries the per-read score records {len, cov, hits, n_best} (SHK_F_SCORES, include/shark_b200.h)."""
         self.lib = capi.load()
         flags = 0 if extend is None else (capi.F_EXTEND_ON if extend else capi.F_EXTEND_OFF)
         if compact:
             flags |= capi.F_COMPACT_RESULTS
         if wide_ids:  # SURVEY.md 8f.4: 32-bit gene ids (more than 65536 reference records), an opt-in extension
             flags |= capi.F_WIDE_IDS
+        if scores:
+            flags |= capi.F_SCORES
         self.compact = bool(compact)
+        self.scores = bool(scores)
         self.wide_ids = bool(wide_ids)
         permille = 0
         if host_pack:  # split upload: part of every chunk is packed to 3 bits per base by the host cores
@@ -255,7 +259,8 @@ class Shark:
 
     def collect(self, slot, copy=True):
         """-> dict(read_idx, gene_idx, keep, gene16, multi, n_probes, n_hits, analyze_ms, ...); with compact=True
-        the expanded arrays (read_idx, gene_idx, keep) are None."""
+        the expanded arrays (read_idx, gene_idx, keep) are None; with scores=True, scores = uint32[n_reads, 4]
+        (len, cov, hits, n_best per read)."""
         res = capi.ChunkResult()
         self._check(self.lib.shk_reads_collect(self.ctx, slot, C.byref(res)))
         n = res.n_assoc
@@ -275,7 +280,17 @@ class Shark:
             keep = np.ctypeslib.as_array(res.keep, shape=(max(res.n_reads, 1),))[: res.n_reads]
             if copy:
                 a, keep = a.copy(), keep.copy()
-        return dict(read_idx=None if a is None else a[:, 0], gene_idx=None if a is None else a[:, 1], keep=keep,
+        scores = None
+        if self.scores:
+            sp, ns = C.POINTER(capi.ReadScore)(), C.c_uint32()
+            self._check(self.lib.shk_reads_scores(self.ctx, slot, C.byref(sp), C.byref(ns)))
+            if ns.value:
+                scores = np.ctypeslib.as_array(C.cast(sp, C.POINTER(C.c_uint32)), shape=(ns.value, 4))
+                if copy:
+                    scores = scores.copy()
+            else:
+                scores = np.zeros((0, 4), np.uint32)
+        return dict(read_idx=None if a is None else a[:, 0], gene_idx=None if a is None else a[:, 1], keep=keep, scores=scores,
                     gene16=gene16, multi=multi, n_multi=int(res.n_multi), n_kept=int(res.n_kept),
                     n_assoc=int(n), n_reads=res.n_reads,
                     n_slow_reads=res.n_slow_reads, n_probes=res.n_probes, n_hits=res.n_hits,
@@ -361,7 +376,8 @@ class Shark:
     def analyze(self, seq, off, qual=None, packed=False):
         """Classifies reads given as SoA (seq uint8, off uint64/uint32 [n+1], qual uint8|None):
         chunks them, streams the chunks through the slots (pinned staging, double buffered) and
-        returns (keep uint8[n], assoc_read uint64[m], assoc_gene uint32[m], stats).  packed=True: every
+        returns (keep uint8[n], assoc_read uint64[m], assoc_gene uint32[m], stats); with scores=True
+        stats["scores"] = uint32[n, 4].  packed=True: every
         chunk is reduced to codes + validity bits with shk_host_pack first and goes through
         shk_reads_submit_packed (what the CLI's batcher does)."""
         seq = np.ascontiguousarray(seq, dtype=np.uint8)
@@ -371,7 +387,7 @@ class Shark:
         if with_qual and qual is None:
             raise capi.SharkError(-1, "min_quality != 0 needs qualities")
         keep = np.zeros(n, np.uint8)
-        out_r, out_g = [], []
+        out_r, out_g, out_s = [], [], []
         stats = dict(n_probes=0, n_hits=0, analyze_ms=0.0, probe_kernel_ms=0.0, n_slow_reads=0, kernel_launches=0, chunks=0,
                      n_extended=0, n_table_loads=0)
         chunks = self.plan_chunks(off) if n else []
@@ -386,6 +402,8 @@ class Shark:
             keep[first:first + r["n_reads"]] = r["keep"]
             out_r.append(r["read_idx"].astype(np.uint64) + np.uint64(first))
             out_g.append(r["gene_idx"])
+            if self.scores:
+                out_s.append(r["scores"])
             for key in ("n_probes", "n_hits", "analyze_ms", "probe_kernel_ms", "n_slow_reads", "kernel_launches",
                         "n_extended", "n_table_loads"):
                 stats[key] += r[key]
@@ -419,6 +437,8 @@ class Shark:
             drain()
         ar = np.concatenate(out_r) if out_r else np.zeros(0, np.uint64)
         ag = np.concatenate(out_g) if out_g else np.zeros(0, np.uint32)
+        if self.scores:  # per read {len, cov, hits, n_best}, in read order
+            stats["scores"] = np.concatenate(out_s) if out_s else np.zeros((0, 4), np.uint32)
         return keep, ar, ag, stats
 
     def analyze_chunks(self, chunks, copy=True, on_result=None, packed=False):
