@@ -267,11 +267,8 @@ __device__ __forceinline__ void window_kmers(uint64_t lo, uint64_t hi, uint32_t 
 // One queued table load per lane: the position's ids go back to the owner of the window; a plain hit of an owner that
 // is looking for a diagonal is verified against the reference (the slot's anchor names a reference window with the
 // same filter bit; it gives a diagonal only if that window IS the read's window, either strand).
-#ifndef SHK_BULK_SERVE_ATTR
-#define SHK_BULK_SERVE_ATTR __forceinline__
-#endif
 template <int MOD>
-__device__ SHK_BULK_SERVE_ATTR void serve_queue(const ReadKernelArgs &a, BulkWarp &sh, uint32_t slot, bool valid, uint32_t want,
+__device__ __forceinline__ void serve_queue(const ReadKernelArgs &a, BulkWarp &sh, uint32_t slot, bool valid, uint32_t want,
                                             uint32_t k, uint64_t kmask2, uint64_t pol_front, uint64_t pol_last)
 {
     if (!valid) return;
@@ -634,19 +631,7 @@ analyze_bulk_kernel(const ReadKernelArgs a)
         }
         a.rec[r] = make_uint2(count, payload);
     }
-    const uint32_t wa = __reduce_add_sync(kFull, count), wp = __reduce_add_sync(kFull, sh.n_probes[lane]),
-                   wh = __reduce_add_sync(kFull, sh.n_hits[lane]), wm = __reduce_add_sync(kFull, multi_entries(count, payload)),
-                   wk = __popc(__ballot_sync(kFull, count != 0u)), we = __reduce_add_sync(kFull, sh.n_ext[lane]),
-                   wl = __reduce_add_sync(kFull, my_loads);
-    if (lane == 0) {
-        if (wm) atomicAdd(&a.tile_sums[tile], wm);
-        if (wa) atomicAdd(&a.counters->n_assoc, (unsigned long long)wa);
-        if (wk) atomicAdd(&a.counters->n_kept, (unsigned long long)wk);
-        if (wp) atomicAdd(&a.counters->n_probes, (unsigned long long)wp);
-        if (wh) atomicAdd(&a.counters->n_hits, (unsigned long long)wh);
-        if (we) atomicAdd(&a.counters->n_extended, (unsigned long long)we);
-        if (wl) atomicAdd(&a.counters->n_table_loads, (unsigned long long)wl);
-    }
+    flush_warp_counters<true>(a, tile, lane, count, payload, sh.n_probes[lane], sh.n_hits[lane], sh.n_ext[lane], my_loads);
 }
 
 // SHK_BULK=1 sends packed reads to this kernel, SHK_BULK=0 keeps them on analyze_reads_kernel<EXT, PACKED> (A/B

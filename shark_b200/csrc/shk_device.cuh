@@ -280,11 +280,7 @@ __device__ __forceinline__ uint4 ld_front(const uint4 *p, uint64_t pol)
 __device__ __forceinline__ uint32_t ld_text_word(const uint32_t *p, uint64_t pol_evict_first)
 {
     uint32_t r;
-#if defined(SHK_TEXT_HINT) && SHK_TEXT_HINT == 0
-    asm volatile("ld.global.nc.u32 %0, [%1];" : "=r"(r) : "l"(p));
-#else
     asm volatile("ld.global.nc.L2::cache_hint.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "l"(pol_evict_first));
-#endif
     return r;
 }
 

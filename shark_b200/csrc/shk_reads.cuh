@@ -1,5 +1,6 @@
 // Pieces shared by the classification kernels (shk_reads.cu, shk_bulk.cu): the register-resident per-gene table of
-// the thread-per-read kernels and the end of a read (arg-max, threshold, -s).  Citations are reference file:line.
+// the thread-per-read kernels, the reporting rule (threshold, -s), the end of a read (arg-max, rule) and the counter
+// flush of the thread-per-read kernels.  Citations are reference file:line.
 #pragma once
 #include "shk_internal.h"
 
@@ -76,7 +77,16 @@ struct Mru4 {
     }
 };
 
-// argmax with ties (ReadAnalyzer.hpp:90-102), threshold and -s (ReadAnalyzer.hpp:104): -> {count, gene | pool offset},
+// Threshold and -s (ReadAnalyzer.hpp:104) for a read whose best genes have coverage `cov` and number `n_best`: is it
+// reported (with n_best associations)?  This is the rule the score records promise (INTEGRATION.md §3); `c * len` is
+// rounded as the reference's double product.  (No test of cov > 0: every gene in a table has cov >= k >= 1, so
+// n_best > 0 implies it.)
+__device__ __forceinline__ bool read_reported(const ReadKernelArgs &a, uint32_t cov, uint32_t len, uint32_t n_best)
+{
+    return n_best > 0 && (double)cov >= __dmul_rn(a.c, (double)len) && (!a.single || n_best == 1);
+}
+
+// argmax with ties (ReadAnalyzer.hpp:90-102), then read_reported: -> {count, gene | pool offset},
 // and the read's score record {len, cov, hits, n_best} (SHK_F_SCORES; dead code for the kernels that do not store it)
 __device__ __forceinline__ void finish_read(const ReadKernelArgs &a, const Mru4 &tab, uint32_t len, uint32_t &count,
                                             uint32_t &payload, uint4 &score)
@@ -99,8 +109,7 @@ __device__ __forceinline__ void finish_read(const ReadKernelArgs &a, const Mru4 
         count += is ? 1u : 0u;
     }
     score = make_uint4(len, maxc, maxh, count);
-    const bool pass = count > 0 && (double)maxc >= __dmul_rn(a.c, (double)len) && (!a.single || count == 1);
-    if (!pass) count = 0;
+    if (!read_reported(a, maxc, len, count)) count = 0;
     if (count == 1) {
         payload = min(min(wg[0], wg[1]), min(wg[2], wg[3]));
     } else if (count >= 2) {
@@ -116,6 +125,33 @@ __device__ __forceinline__ void finish_read(const ReadKernelArgs &a, const Mru4 
 #pragma unroll
             for (int i = 0; i < 4; ++i)
                 if ((uint32_t)i < count) a.pool[payload + i] = wg[i];
+        }
+    }
+}
+
+// End of the thread-per-read kernels (K6, K6b): the warp's reads go into the chunk's counters and its multi entries into
+// tile_sums, which is zeroed before the launch.  Every warp retires on its own: no warp of a CTA waits at a barrier for
+// its slowest sibling.  EXT: also the anchor-and-extend counters.
+template <bool EXT>
+__device__ __forceinline__ void flush_warp_counters(const ReadKernelArgs &a, uint32_t tile, int lane, uint32_t count,
+                                                    uint32_t payload, uint32_t probes, uint32_t hits, uint32_t ext,
+                                                    uint32_t loads)
+{
+    const uint32_t wa = __reduce_add_sync(kFull, count), wp = __reduce_add_sync(kFull, probes),
+                   wh = __reduce_add_sync(kFull, hits), wm = __reduce_add_sync(kFull, multi_entries(count, payload)),
+                   wk = __popc(__ballot_sync(kFull, count != 0u));
+    if (lane == 0) {
+        if (wm) atomicAdd(&a.tile_sums[tile], wm);
+        if (wa) atomicAdd(&a.counters->n_assoc, (unsigned long long)wa);
+        if (wk) atomicAdd(&a.counters->n_kept, (unsigned long long)wk);
+        if (wp) atomicAdd(&a.counters->n_probes, (unsigned long long)wp);
+        if (wh) atomicAdd(&a.counters->n_hits, (unsigned long long)wh);
+    }
+    if (EXT) {
+        const uint32_t we = __reduce_add_sync(kFull, ext), wl = __reduce_add_sync(kFull, loads);
+        if (lane == 0) {
+            if (we) atomicAdd(&a.counters->n_extended, (unsigned long long)we);
+            if (wl) atomicAdd(&a.counters->n_table_loads, (unsigned long long)wl);
         }
     }
 }
