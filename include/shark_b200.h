@@ -89,6 +89,11 @@ typedef struct shk_params {
  * so that a caller can classify a sample once and apply any -c and -s afterwards (INTEGRATION.md 3).  16 bytes per
  * read more cross the link; without the flag nothing is written, allocated or copied. */
 #define SHK_F_SCORES 32u
+/* Count reads per gene on the device (shk_gene_counts): every chunk's reported associations are added into two 64-bit
+ * counters per gene index that stay on the device, so that a caller gets the per-gene table of a whole sample without
+ * walking gene16 / multi (INTEGRATION.md 3).  One more kernel launch per chunk; without the flag nothing is launched or
+ * allocated. */
+#define SHK_F_GENE_COUNTS 128u
 
 /* Compact per-read result words (shk_chunk_result.gene16). */
 #define SHK_GENE_NONE 0xFFFFu  /* no association: the read is not reported                                */
@@ -176,6 +181,19 @@ typedef struct shk_read_score {
  * memory, valid until the slot's next submit (same lifetime as gene16).  A read without a window of k valid bases
  * gets {len, 0, 0, 0}.  SHK_E_STATE for a context created without SHK_F_SCORES or before the slot is collected. */
 int shk_reads_scores(shk_ctx *ctx, uint32_t slot, const shk_read_score **scores, uint32_t *n_reads);
+
+/* Per-gene read counts (SHK_F_GENE_COUNTS), for every gene index g in [0, n_genes):
+ *     unique[g]  reported reads whose only association is g (a single winner whose index is SHK_GENE_MULTI or
+ *                SHK_GENE_NONE travels through `multi` but counts here)
+ *     shared[g]  reported reads that have g among two or more tied associations
+ * so that unique[g] + shared[g] = the associations {read, g} that shk_reads_collect returned, under the context's -c,
+ * -s and -q.  Every chunk adds to the counters once, including chunks that shk_reads_collect had to run again, and
+ * every shk_reads_analyze_resident adds again (the same resident chunk analysed n times counts n times).  The counters
+ * are zeroed whenever an index becomes ready and by shk_gene_counts_reset.  n must equal shk_index_info.n_genes;
+ * either pointer may be NULL.  SHK_E_STATE for a context created without the flag, without an index, or while a slot
+ * has an uncollected chunk.  The read-back counts in shk_d2h_bytes. */
+int shk_gene_counts(shk_ctx *ctx, uint64_t *unique, uint64_t *shared, uint32_t n);
+int shk_gene_counts_reset(shk_ctx *ctx);
 
 /* ---- lifetime ------------------------------------------------------------------------ */
 
@@ -407,7 +425,7 @@ int shk_upload_stats(const shk_ctx *ctx, double *packed_share, double *pack_gbas
 
 /* Bytes that shk_reads_submit / shk_reads_upload copied host -> device on this context so far. */
 uint64_t shk_h2d_bytes(const shk_ctx *ctx);
-/* Result bytes (associations, keep flags, counters, score records) copied device -> host on this context so far.  The
+/* Result bytes (associations, keep flags, counters, score records, gene counts) copied device -> host on this context so far.  The
  * read-back of a chunk is enqueued with its kernels, sized by the previous chunks' associations per read;
  * shk_reads_collect fetches what that did not cover. */
 uint64_t shk_d2h_bytes(const shk_ctx *ctx);

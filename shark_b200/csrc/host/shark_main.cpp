@@ -10,7 +10,9 @@
 // the gene names still come from -r), --wide-ids (32-bit gene ids: references of more than 65536 records, which
 // the reference's 16-bit ids cannot index - small_vector.hpp:46; without the flag such inputs end with an error),
 // --scores FILE (one line `<name> <len> <cov> <hits> <n_best>` per reported read, in the order of the ssv: the numbers
-// behind each answer, from which any -c / -s can be applied afterwards - shk_read_score, include/shark_b200.h).
+// behind each answer, from which any -c / -s can be applied afterwards - shk_read_score, include/shark_b200.h),
+// --counts FILE (one line `<name> <unique> <shared>` per gene index, in index order: the run's reported reads counted
+// per gene on the device - shk_gene_counts, include/shark_b200.h; <name> is the ssv's name of that index).
 //
 // Pipeline (pipeline.hpp, fastpipe.hpp, ingest.hpp): plain input files are memory-mapped and scanned by
 // the host pool in parallel (compressed ones by a streaming scanner per file); a batcher thread turns runs
@@ -86,6 +88,7 @@ struct Options {
     bool wide_ids = false;          // extension: more than 65536 reference records (SHK_F_WIDE_IDS)
     std::string save_index, load_index;  // extensions
     std::string scores_path;        // extension: per-read score records (SHK_F_SCORES)
+    std::string counts_path;        // extension: per-gene read counts (SHK_F_GENE_COUNTS)
 };
 
 [[noreturn]] void usage_error(const char *msg, bool with_usage)
@@ -158,6 +161,7 @@ const OptionRow kOptions[] = {
     {1004, "load-index", true, [](Options &o, std::istringstream &a) { a >> o.load_index; }},
     {1005, "wide-ids", false, [](Options &o, std::istringstream &) { o.wide_ids = true; }},
     {1006, "scores", true, [](Options &o, std::istringstream &a) { a >> o.scores_path; }},
+    {1007, "counts", true, [](Options &o, std::istringstream &a) { a >> o.counts_path; }},
 };
 
 Options parse_arguments(int argc, char **argv)
@@ -291,8 +295,11 @@ private:
 //     finishes on its own ("detached tear-down").
 // The two share one anonymous mapping created before the fork: per chunk buffer a slot with the packed chunk
 // (offsets, code words, validity words; host -> device) and the compact results (one 16-bit word per read + the
-// list for ties, and with --scores the score records, 16 bytes per read; device -> host).  Two pipes carry the small messages.  SHK_ONE_PROCESS=1 runs the device side as
-// a thread of the host process instead (same protocol; for debuggers and sanitizers).
+// list for ties, and with --scores the score records, 16 bytes per read; device -> host).  With --counts one more
+// region after the slots receives the per-gene table of the whole run (device -> host, once, before kMsgDone): it is
+// sized for the largest gene index count the run can have, 65536 (16-bit ids) or kMaxCountGenes (--wide-ids), and a
+// reference with more fails before the first chunk.  Two pipes carry the small messages.  SHK_ONE_PROCESS=1 runs the
+// device side as a thread of the host process instead (same protocol; for debuggers and sanitizers).
 // ---------------------------------------------------------------------------------------------------------
 struct SlotView {
     uint32_t *off;
@@ -302,13 +309,16 @@ struct SlotView {
     shkhost::AssocPair *multi;
     uint32_t *scores;  // nullptr without --scores
 };
+constexpr uint32_t kMaxCountGenes = 1u << 24;  // --counts --wide-ids: 256 MiB of address space, touched as far as used
 struct SharedLayout {
     char *base = nullptr;
     size_t n_slots = 0, slot_bytes = 0;
     size_t off_bytes = 0, codes_bytes = 0, valid_bytes = 0, gene_bytes = 0, multi_cap = 0, scores_bytes = 0;
+    size_t counts_cap = 0;  // --counts: gene indices the table after the slots holds (0: no table)
     static size_t round(size_t n) { return (n + 4095) / 4096 * 4096; }
-    void plan(size_t slots, size_t max_reads, uint64_t max_bytes, bool scores)
+    void plan(size_t slots, size_t max_reads, uint64_t max_bytes, bool scores, size_t count_genes)
     {
+        counts_cap = count_genes;
         n_slots = slots;
         const size_t groups = (size_t)((max_bytes + 31) / 32) + 2;
         off_bytes = round((max_reads + 2) * 4);
@@ -321,7 +331,7 @@ struct SharedLayout {
     }
     bool map()
     {
-        void *m = mmap(nullptr, n_slots * slot_bytes, PROT_READ | PROT_WRITE, MAP_SHARED | MAP_ANONYMOUS | MAP_NORESERVE, -1, 0);
+        void *m = mmap(nullptr, n_slots * slot_bytes + counts_cap * 2 * sizeof(uint64_t), PROT_READ | PROT_WRITE, MAP_SHARED | MAP_ANONYMOUS | MAP_NORESERVE, -1, 0);
         if (m == MAP_FAILED) return false;
         base = (char *)m;
         return true;
@@ -338,6 +348,8 @@ struct SharedLayout {
         v.scores = scores_bytes ? (uint32_t *)(p + slot_bytes - scores_bytes) : nullptr;
         return v;
     }
+    // --counts: unique[n_genes] then shared[n_genes] (shk_gene_counts)
+    uint64_t *counts() const { return (uint64_t *)(base + n_slots * slot_bytes); }
 };
 
 enum : uint32_t { kMsgChunk = 1, kMsgEnd = 2, kMsgReady = 3, kMsgResult = 4, kMsgDone = 5 };
@@ -422,7 +434,8 @@ void device_main(const Options &opt, const SharedLayout &shm, unsigned chunk_rea
         p.n_slots = 2;
         p.max_reads_per_chunk = chunk_reads;
         p.max_bytes_per_chunk = max_chunk_bytes;
-        p.flags = SHK_F_COMPACT_RESULTS | (opt.wide_ids ? SHK_F_WIDE_IDS : 0u) | (opt.scores_path.empty() ? 0u : SHK_F_SCORES);
+        p.flags = SHK_F_COMPACT_RESULTS | (opt.wide_ids ? SHK_F_WIDE_IDS : 0u) | (opt.scores_path.empty() ? 0u : SHK_F_SCORES) |
+                  (shm.counts_cap ? SHK_F_GENE_COUNTS : 0u);
         if (shk_create(&p, &ctxs[g]) != SHK_OK) die(std::string("shk_create: ") + shk_last_error(nullptr));
     }
     tstamp("contexts created");
@@ -448,6 +461,9 @@ void device_main(const Options &opt, const SharedLayout &shm, unsigned chunk_rea
     if (!replicated)
         for (int g = 1; g < opt.gpus; ++g) SHK_TRY(ctxs[g], shk_index_replicate(ctxs[0], ctxs[g]));
     tstamp("index ready");
+    if (shm.counts_cap && info.n_genes > shm.counts_cap)
+        die("--counts: the reference has " + std::to_string(info.n_genes) + " gene indices, the count table holds " +
+            std::to_string(shm.counts_cap));
     std::vector<uint8_t>().swap(ref_bases);
     Msg ready;
     ready.kind = kMsgReady;
@@ -506,10 +522,21 @@ void device_main(const Options &opt, const SharedLayout &shm, unsigned chunk_rea
     }
     while (!inflight.empty()) drain_one();
     tstamp("last chunk collected");
+    if (shm.counts_cap) {  // --counts: the run's table, summed over the GPUs, into the shared region
+        const uint32_t n = info.n_genes;
+        uint64_t *tab = shm.counts();
+        std::vector<uint64_t> u(n), s(n);
+        memset(tab, 0, (size_t)n * 2 * sizeof(uint64_t));
+        for (shk_ctx *c : ctxs) {
+            SHK_TRY(c, shk_gene_counts(c, u.data(), s.data(), n));
+            for (uint32_t g = 0; g < n; ++g) tab[g] += u[g], tab[n + g] += s[g];
+        }
+    }
     if (g_timing) fprintf(stderr, "[shark-b200/timing] device side: %llu chunks, submit %.0f ms, collect %.0f ms\n",
                           (unsigned long long)submitted, t_submit * 1e3, t_collect * 1e3);
     Msg d;
     d.kind = kMsgDone;
+    d.n_genes = info.n_genes;
     write_all(out, &d, sizeof d);
     if (getenv("SHK_CLEAN_EXIT")) {
         for (auto *c : ctxs) shk_destroy(c);
@@ -556,7 +583,8 @@ int main(int argc, char *argv[])
         close(fd);
     }
     SharedLayout shm;
-    shm.plan(n_bufs, chunk_reads, max_chunk_bytes, !opt.scores_path.empty());
+    shm.plan(n_bufs, chunk_reads, max_chunk_bytes, !opt.scores_path.empty(),
+             opt.counts_path.empty() ? 0 : opt.wide_ids ? kMaxCountGenes : 65536);
     if (!shm.map()) die("cannot map the chunk buffers");
     int h2d[2], d2h[2];
     if (pipe(h2d) != 0 || pipe(d2h) != 0) die("cannot create pipes");
@@ -662,6 +690,8 @@ int main(int argc, char *argv[])
     const int fd2 = (!opt.paired || opt.out2_path.empty()) ? -1 : open(opt.out2_path.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0666);
     const int fd_scores = opt.scores_path.empty() ? -1 : open(opt.scores_path.c_str(), O_RDWR | O_CREAT | O_TRUNC, 0666);
     if (!opt.scores_path.empty() && fd_scores < 0) die("cannot create " + opt.scores_path);
+    const int fd_counts = opt.counts_path.empty() ? -1 : open(opt.counts_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0666);
+    if (!opt.counts_path.empty() && fd_counts < 0) die("cannot create " + opt.counts_path);
     Writer writer(STDOUT_FILENO, fd1, fd2, legend_ID, opt.paired, fd_scores);
     if (!(getenv("SHK_PREFAULT") && atoi(getenv("SHK_PREFAULT")) == 0)) {
         // the filtered FASTQ of a FASTQ sample is never longer than the sample (pipeline.hpp, Writer::start_prefault)
@@ -685,6 +715,7 @@ int main(int argc, char *argv[])
 
     // results, in the order the chunks were sent
     uint64_t total_reads = 0, chunks_done = 0;
+    uint32_t n_genes = 0;
     bool got_ready = false, got_done = false;
     for (;;) {
         Msg m;
@@ -699,6 +730,7 @@ int main(int argc, char *argv[])
         }
         if (m.kind == kMsgDone) {
             got_done = true;
+            n_genes = m.n_genes;
             break;
         }
         if (m.kind != kMsgResult || m.slot >= n_bufs) break;
@@ -730,6 +762,19 @@ int main(int argc, char *argv[])
     if (fd1 >= 0) close(fd1);
     if (fd2 >= 0) close(fd2);
     if (fd_scores >= 0) close(fd_scores);
+    if (fd_counts >= 0) {  // `<name> <unique> <shared>` per gene index, the name as the ssv prints it
+        const uint64_t *tab = shm.counts();
+        std::string txt;
+        for (uint32_t g = 0; g < n_genes; ++g) {
+            if (g < legend_ID.size()) txt += legend_ID[g];
+            txt += ' ';
+            txt += std::to_string(tab[g]);
+            txt += ' ';
+            txt += std::to_string(tab[n_genes + g]);
+            txt += '\n';
+        }
+        if (!write_all(fd_counts, txt.data(), txt.size()) || close(fd_counts) != 0) die("cannot write " + opt.counts_path);
+    }
     tstamp("output written");
     if (g_timing) {
         const shkhost::StageTimes &st = shkhost::stage_times();

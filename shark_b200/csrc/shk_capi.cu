@@ -291,6 +291,25 @@ static int ensure_slow_table(shk_ctx *ctx)
         SHK_CUDA(ctx, cudaMemset(s.d_slow_table, 0, slabs * ng * sizeof(uint4)));
         SHK_CUDA(ctx, cudaMemset(s.d_slow_stamp, 0, slabs * 4));
     }
+    if (ctx->gene_counts) {  // the counts of the new index start at zero
+        cudaFree(ctx->d_gene_counts);
+        ctx->d_gene_counts = nullptr;
+        SHK_CUDA(ctx, cudaMalloc((void **)&ctx->d_gene_counts, 2 * ng * sizeof(unsigned long long)));
+        SHK_CUDA(ctx, cudaMemsetAsync(ctx->d_gene_counts, 0, 2 * ng * sizeof(unsigned long long), ctx->build_stream));
+        SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
+    }
+    return SHK_OK;
+}
+
+// shk_gene_counts / shk_gene_counts_reset: the counters exist and no chunk is adding to them
+static int gene_counts_guard(shk_ctx *ctx)
+{
+    if (!ctx) return fail(nullptr, SHK_E_ARG, "NULL context");
+    if (!ctx->gene_counts) return fail(ctx, SHK_E_STATE, "the context was created without SHK_F_GENE_COUNTS");
+    if (!ctx->index.built || !ctx->d_gene_counts) return fail(ctx, SHK_E_STATE, "no index");
+    for (uint32_t i = 0; i < ctx->n_slots; ++i)
+        if (ctx->slots[i].pending) return fail(ctx, SHK_E_STATE, "slot %u has an uncollected chunk: call shk_reads_collect first", i);
+    SHK_CUDA(ctx, cudaSetDevice(ctx->device));
     return SHK_OK;
 }
 
@@ -496,7 +515,8 @@ int shk_create(const shk_params *p, shk_ctx **out)
     if (p->bf_bits < 64) return fail(nullptr, SHK_E_ARG, "bf_bits must be >= 64");
     if ((p->flags & SHK_F_EXTEND_ON) && (p->flags & SHK_F_EXTEND_OFF))
         return fail(nullptr, SHK_E_ARG, "SHK_F_EXTEND_ON and SHK_F_EXTEND_OFF are exclusive");
-    if (p->flags & ~(SHK_F_EXTEND_ON | SHK_F_EXTEND_OFF | SHK_F_HOST_PACK | SHK_F_COMPACT_RESULTS | SHK_F_WIDE_IDS | SHK_F_SCORES))
+    if (p->flags & ~(SHK_F_EXTEND_ON | SHK_F_EXTEND_OFF | SHK_F_HOST_PACK | SHK_F_COMPACT_RESULTS | SHK_F_WIDE_IDS | SHK_F_SCORES |
+                     SHK_F_GENE_COUNTS))
         return fail(nullptr, SHK_E_ARG, "unknown flag bits");
     if ((p->flags & SHK_F_WIDE_IDS) && (p->flags & SHK_F_EXTEND_ON))
         return fail(nullptr, SHK_E_ARG, "SHK_F_WIDE_IDS has no extension structures (SHK_F_EXTEND_ON)");
@@ -521,6 +541,7 @@ int shk_create(const shk_params *p, shk_ctx **out)
     ctx->compact_results = (p->flags & SHK_F_COMPACT_RESULTS) != 0;
     ctx->wide_ids = (p->flags & SHK_F_WIDE_IDS) != 0;
     ctx->scores = (p->flags & SHK_F_SCORES) != 0;
+    ctx->gene_counts = (p->flags & SHK_F_GENE_COUNTS) != 0;
     if (const char *ev = getenv("SHK_HOST_PACK")) ctx->host_pack = atoi(ev) != 0;  // tuning override
     int rc = SHK_OK;
     auto bail = [&](int code) {
@@ -599,6 +620,7 @@ void shk_destroy(shk_ctx *ctx)
     cudaFree(ctx->index.refr);
     cudaFree(ctx->index.ebits);
     cudaFree(ctx->index.front_plain);
+    cudaFree(ctx->d_gene_counts);
     if (ctx->build_stream) cudaStreamDestroy(ctx->build_stream);
     if (ctx->ev_t0) cudaEventDestroy(ctx->ev_t0);
     if (ctx->ev_t1) cudaEventDestroy(ctx->ev_t1);
@@ -1276,6 +1298,33 @@ int shk_reads_scores(shk_ctx *ctx, uint32_t slot, const shk_read_score **scores,
     if (!s.collected) return fail(ctx, SHK_E_STATE, "slot %u has no collected chunk", slot);
     *scores = s.h_scores;
     *n_reads = s.n_reads;
+    return SHK_OK;
+}
+
+int shk_gene_counts(shk_ctx *ctx, uint64_t *unique, uint64_t *shared, uint32_t n)
+{
+    int rc = gene_counts_guard(ctx);
+    if (rc) return rc;
+    const uint32_t ng = ctx->index.info.n_genes;
+    if (n != ng) return fail(ctx, SHK_E_ARG, "n = %u, the index has %u gene indices", n, ng);
+    uint64_t *dst[2] = {unique, shared};
+    for (int h = 0; h < 2; ++h) {
+        if (!dst[h] || !ng) continue;
+        SHK_CUDA(ctx, cudaMemcpyAsync(dst[h], ctx->d_gene_counts + (size_t)h * ng, (size_t)ng * sizeof(uint64_t),
+                                      cudaMemcpyDeviceToHost, ctx->build_stream));
+        ctx->d2h_bytes += (uint64_t)ng * sizeof(uint64_t);
+    }
+    SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
+    return SHK_OK;
+}
+
+int shk_gene_counts_reset(shk_ctx *ctx)
+{
+    int rc = gene_counts_guard(ctx);
+    if (rc) return rc;
+    const uint64_t ng = std::max<uint32_t>(ctx->index.info.n_genes, 1);
+    SHK_CUDA(ctx, cudaMemsetAsync(ctx->d_gene_counts, 0, 2 * ng * sizeof(unsigned long long), ctx->build_stream));
+    SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
     return SHK_OK;
 }
 

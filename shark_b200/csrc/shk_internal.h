@@ -222,6 +222,10 @@ struct shk_ctx {
     bool compact_results = false;          // SHK_F_COMPACT_RESULTS
     bool wide_ids = false;                 // SHK_F_WIDE_IDS
     bool scores = false;                   // SHK_F_SCORES
+    bool gene_counts = false;              // SHK_F_GENE_COUNTS
+    // SHK_F_GENE_COUNTS: [0, n_genes) reads whose only association is g, [n_genes, 2 n_genes) reads with g among tied
+    // associations; (re)allocated and zeroed whenever an index becomes ready, added to by every chunk's K8
+    unsigned long long *d_gene_counts = nullptr;
     shk::PackControl pack;                 // split upload: feedback state of the packed share
     char err[512] = {0};
 };
@@ -266,7 +270,8 @@ void shard_free(shk_ctx *ctx);
 void shard_cuts_host(const uint64_t *rec_off, uint32_t n_rec, uint32_t n_shards, uint64_t *cuts);
 
 // shk_reads.cu
-// Enqueues the classification kernels of one chunk on `st`; returns the number of launches.
+// Enqueues the classification kernels of one chunk on `st` (and K8 when ctx->d_gene_counts exists); returns the number
+// of launches.
 int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t assoc_cap, cudaStream_t st, cudaEvent_t ev_k0,
                         cudaEvent_t ev_ka, cudaEvent_t ev_k1);
 int launch_scatter(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t assoc_cap, cudaStream_t st);

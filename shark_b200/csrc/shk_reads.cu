@@ -13,6 +13,8 @@
 //                          K6m cannot hold (more than kMidMaxGenes genes)
 //   scan_tile_sums_kernel  exclusive scan of the per-tile association counts
 //   scatter_assoc_kernel   ordered (read_idx, gene_idx) list + keep flags
+//   gene_counts_kernel     K8, SHK_F_GENE_COUNTS only: per-gene counts of the chunk's reported reads, added into the
+//                          context's device counters
 #include "shk_internal.h"
 #include "shk_scan.cuh"
 #include "shk_reads.cuh"
@@ -784,6 +786,64 @@ scatter_assoc_kernel(const ReadKernelArgs a, uint64_t multi_cap, const uint32_t 
     if (blockIdx.x == 0 && threadIdx.x == 0) a.counters->n_multi = *total;
 }
 
+// ---------------------------------------------------------------------------------------------
+// K8 (SHK_F_GENE_COUNTS): per-gene counts of the chunk's reported reads, added into counts[0, n_genes) (reads whose only
+// association is g) and counts[n_genes, 2 n_genes) (reads with g among two or more tied associations).  Reads rec and
+// pool once the classification kernels have settled every read, so it counts exactly what the result lists hold, on
+// every path and id width.  No address is hot: the single winners of a warp are merged with __match_any_sync (one add
+// per distinct gene), and the genes of one tied read are distinct, so the warp adds them 32 at a time without a
+// conflict.  SMEM: the adds go to a per-CTA histogram in shared memory, and every non-zero bin reaches global memory
+// once per CTA.  A chunk whose tie pool overflowed adds nothing: the host runs the whole chunk again.
+// ---------------------------------------------------------------------------------------------
+constexpr uint32_t kCountThreads = 256;
+constexpr uint32_t kCountSmemGenes = 6144;  // 2 x 6144 32-bit bins = 48 KB, the most static shared memory a kernel may have
+
+template <bool SMEM>
+__global__ void __launch_bounds__(kCountThreads)
+gene_counts_kernel(const uint2 *__restrict__ rec, const uint32_t *__restrict__ pool, uint32_t n_reads, uint32_t n_genes,
+                   const ChunkCounters *counters, unsigned long long *counts)
+{
+    __shared__ uint32_t hist[SMEM ? 2 * kCountSmemGenes : 1];
+    if (counters->pool_overflow) return;  // the same for every thread of the grid
+    if (SMEM) {
+        for (uint32_t i = threadIdx.x; i < 2 * n_genes; i += kCountThreads) hist[i] = 0;
+        __syncthreads();
+    }
+    auto add = [&](uint32_t bin, uint32_t v) {
+        if (SMEM) atomicAdd(&hist[bin], v);
+        else atomicAdd(&counts[bin], (unsigned long long)v);
+    };
+    const int lane = threadIdx.x & 31;
+    for (uint32_t w = blockIdx.x * kCountThreads + (threadIdx.x & ~31u); w < n_reads; w += gridDim.x * kCountThreads) {
+        const uint32_t r = w + lane;
+        const uint2 rc = r < n_reads ? rec[r] : make_uint2(0u, 0u);
+        const uint32_t g = rc.x == 1u ? rc.y : 0xFFFFFFFFu;  // gene ids are < n_genes < 2^32
+        const uint32_t peers = __match_any_sync(kFull, g);
+        if (g != 0xFFFFFFFFu && lane == __ffs(peers) - 1) add(g, __popc(peers));
+        for (uint32_t tied = __ballot_sync(kFull, rc.x >= 2u); tied; tied &= tied - 1u) {
+            const int src = __ffs(tied) - 1;
+            const uint32_t cnt = __shfl_sync(kFull, rc.x, src), off = __shfl_sync(kFull, rc.y, src);
+            for (uint32_t t = lane; t < cnt; t += 32) add(n_genes + pool[off + t], 1u);
+        }
+    }
+    if (SMEM) {
+        __syncthreads();
+        for (uint32_t i = threadIdx.x; i < 2 * n_genes; i += kCountThreads)
+            if (hist[i]) atomicAdd(&counts[i], (unsigned long long)hist[i]);
+    }
+}
+
+static void launch_gene_counts(shk_ctx *ctx, const ReadKernelArgs &a, cudaStream_t st)
+{
+    const bool smem = a.n_genes <= kCountSmemGenes;
+    const unsigned per_sm = smem ? 4u : 8u;
+    const unsigned blocks = std::min<unsigned>((a.n_reads + kCountThreads - 1) / kCountThreads, (unsigned)ctx->sm_count * per_sm);
+    if (smem)
+        gene_counts_kernel<true><<<blocks, kCountThreads, 0, st>>>(a.rec, a.pool, a.n_reads, a.n_genes, a.counters, ctx->d_gene_counts);
+    else
+        gene_counts_kernel<false><<<blocks, kCountThreads, 0, st>>>(a.rec, a.pool, a.n_reads, a.n_genes, a.counters, ctx->d_gene_counts);
+}
+
 // SHK_F_WIDE_IDS: there is no front table, every read goes to the middle path.
 __global__ void __launch_bounds__(256) all_reads_slow_kernel(const ReadKernelArgs a)
 {
@@ -861,12 +921,13 @@ int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t multi_ca
         cudaMemsetAsync(a.tile_sums, 0, (size_t)tiles * 4, st);  // the classification kernels add to it
         if (a.scores) launch_classify<true>(a, st, tiles, slow_blocks, ev_ka);
         else launch_classify<false>(a, st, tiles, slow_blocks, ev_ka);
+        if (ctx->d_gene_counts) launch_gene_counts(ctx, a, st);
         // tile_base <- exclusive scan(tile_sums); the grand total lands in tile_base[tiles]
         cudaMemcpyAsync(a.tile_base, a.tile_sums, (size_t)tiles * 4, cudaMemcpyDeviceToDevice, st);
         scan_tile_sums_kernel<<<1, 1024, 0, st>>>(a.tile_base, tiles, a.tile_base + tiles);
         scatter_assoc_kernel<<<tiles, kReadsPerTile, 0, st>>>(a, multi_cap, a.tile_base + tiles);
         const uint32_t split = std::min(a.pack_first, a.n_reads);
-        launched = a.wide ? 5 : 4 + (split > 0 ? 1 : 0) + (split < a.n_reads ? 1 : 0);
+        launched = (a.wide ? 5 : 4 + (split > 0 ? 1 : 0) + (split < a.n_reads ? 1 : 0)) + (ctx->d_gene_counts ? 1 : 0);
         ctx->launches += launched;
     }
     else if (ev_ka) cudaEventRecord(ev_ka, st);

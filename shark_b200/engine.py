@@ -16,11 +16,13 @@ from . import capi
 class Shark:
     def __init__(self, k=17, c=0.6, bf_bits=1 << 33, min_quality=0, single=False, device=0, n_slots=2,
                  max_reads_per_chunk=1 << 20, max_bytes_per_chunk=0, extend=None, host_pack=False, compact=False,
-                 wide_ids=False, scores=False):
+                 wide_ids=False, scores=False, gene_counts=False):
         """extend: None = automatic (anchor-and-extend when the front table is DRAM-sized), True /
         False = force it on / off (results are identical; tests run both).  compact: results stay in the
         compact form (gene16 / multi), shk_reads_collect does no per-read host work.  scores: every result also
-        carries the per-read score records {len, cov, hits, n_best} (SHK_F_SCORES, include/shark_b200.h)."""
+        carries the per-read score records {len, cov, hits, n_best} (SHK_F_SCORES, include/shark_b200.h).
+        gene_counts: every chunk's reported reads are also counted per gene on the device (SHK_F_GENE_COUNTS);
+        gene_counts() reads the table back."""
         self.lib = capi.load()
         flags = 0 if extend is None else (capi.F_EXTEND_ON if extend else capi.F_EXTEND_OFF)
         if compact:
@@ -29,6 +31,8 @@ class Shark:
             flags |= capi.F_WIDE_IDS
         if scores:
             flags |= capi.F_SCORES
+        if gene_counts:
+            flags |= capi.F_GENE_COUNTS
         self.compact = bool(compact)
         self.scores = bool(scores)
         self.wide_ids = bool(wide_ids)
@@ -256,6 +260,18 @@ class Shark:
 
     def analyze_resident(self, slot):
         self._check(self.lib.shk_reads_analyze_resident(self.ctx, slot))
+
+    def gene_counts(self):
+        """-> (unique, shared), uint64[n_genes] each: reported reads whose only association is gene g, and reported
+        reads with g among two or more tied associations, summed over every chunk since the index became ready or
+        the last reset_gene_counts() (shk_gene_counts; needs gene_counts=True and every submitted chunk collected)."""
+        n = self.info.n_genes if self.info is not None else 0
+        unique, shared = np.zeros(n, np.uint64), np.zeros(n, np.uint64)
+        self._check(self.lib.shk_gene_counts(self.ctx, capi.ptr(unique), capi.ptr(shared), n))
+        return unique, shared
+
+    def reset_gene_counts(self):
+        self._check(self.lib.shk_gene_counts_reset(self.ctx))
 
     def collect(self, slot, copy=True):
         """-> dict(read_idx, gene_idx, keep, gene16, multi, n_probes, n_hits, analyze_ms, ...); with compact=True
