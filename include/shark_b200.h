@@ -94,6 +94,11 @@ typedef struct shk_params {
  * walking gene16 / multi (INTEGRATION.md 3).  One more kernel launch per chunk; without the flag nothing is launched or
  * allocated. */
 #define SHK_F_GENE_COUNTS 128u
+/* Count reads per equivalence class on the device (shk_eq_classes): the set of genes a reported read is associated
+ * with, and the number of reads with exactly that set, over a whole sample (INTEGRATION.md 3).  Needs
+ * SHK_F_GENE_COUNTS (the singleton classes are its `unique` counters).  The insert pass runs inside K8; a device hash
+ * table grows as classes appear.  Without the flag nothing is launched, allocated or copied. */
+#define SHK_F_EQ_CLASSES 512u
 
 /* Compact per-read result words (shk_chunk_result.gene16). */
 #define SHK_GENE_NONE 0xFFFFu  /* no association: the read is not reported                                */
@@ -189,11 +194,25 @@ int shk_reads_scores(shk_ctx *ctx, uint32_t slot, const shk_read_score **scores,
  * so that unique[g] + shared[g] = the associations {read, g} that shk_reads_collect returned, under the context's -c,
  * -s and -q.  Every chunk adds to the counters once, including chunks that shk_reads_collect had to run again, and
  * every shk_reads_analyze_resident adds again (the same resident chunk analysed n times counts n times).  The counters
- * are zeroed whenever an index becomes ready and by shk_gene_counts_reset.  n must equal shk_index_info.n_genes;
+ * are zeroed whenever an index becomes ready and by shk_gene_counts_reset, which with SHK_F_EQ_CLASSES also empties the
+ * class table (its singletons are these counters).  n must equal shk_index_info.n_genes;
  * either pointer may be NULL.  SHK_E_STATE for a context created without the flag, without an index, or while a slot
  * has an uncollected chunk.  The read-back counts in shk_d2h_bytes. */
 int shk_gene_counts(shk_ctx *ctx, uint64_t *unique, uint64_t *shared, uint32_t n);
 int shk_gene_counts_reset(shk_ctx *ctx);
+
+/* Reads per equivalence class (SHK_F_EQ_CLASSES).  A reported read's class is the set of its n_best associations in
+ * ascending gene index order, under the context's -c, -s and -q; class i is ids[offsets[i], offsets[i+1]) and
+ * counts[i] reads had exactly that set.  Classes come in lexicographic order of their id lists; singletons are
+ * included ({g} counts unique[g] of shk_gene_counts), classes with no read are not.  So the classes containing g add up
+ * to unique[g] + shared[g], and the counts to the n_kept of the chunks.  Accumulation and reset are those of
+ * shk_gene_counts: every chunk adds once, every shk_reads_analyze_resident adds again, and the table is emptied
+ * whenever an index becomes ready and by shk_gene_counts_reset.  Two calls: with NULL arrays only *n_classes and
+ * *n_ids are set; then arrays of n_classes + 1, n_ids and n_classes entries (cap_classes >= n_classes, cap_ids >= n_ids,
+ * SHK_E_CAPACITY otherwise, with the sizes set; ids and counts may be NULL when they would be empty).  SHK_E_STATE for a context created without the flag, without an index,
+ * or while a slot has an uncollected chunk.  The read-back counts in shk_d2h_bytes. */
+int shk_eq_classes(shk_ctx *ctx, uint64_t *n_classes, uint64_t *n_ids, uint64_t *offsets, uint32_t *ids, uint64_t *counts,
+                   uint64_t cap_classes, uint64_t cap_ids);
 
 /* ---- lifetime ------------------------------------------------------------------------ */
 
@@ -425,7 +444,7 @@ int shk_upload_stats(const shk_ctx *ctx, double *packed_share, double *pack_gbas
 
 /* Bytes that shk_reads_submit / shk_reads_upload copied host -> device on this context so far. */
 uint64_t shk_h2d_bytes(const shk_ctx *ctx);
-/* Result bytes (associations, keep flags, counters, score records, gene counts) copied device -> host on this context so far.  The
+/* Result bytes (associations, keep flags, counters, score records, gene counts, class tables) copied device -> host on this context so far.  The
  * read-back of a chunk is enqueued with its kernels, sized by the previous chunks' associations per read;
  * shk_reads_collect fetches what that did not cover. */
 uint64_t shk_d2h_bytes(const shk_ctx *ctx);

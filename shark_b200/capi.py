@@ -26,7 +26,7 @@ EXPORTED = [
     "shk_shard_finish", "shk_shard_end", "shk_shard_cuts", "shk_index_build_sharded", "shk_index_save", "shk_index_load",
     "shk_host_pack", "shk_host_pack_info", "shk_h2d_bytes", "shk_d2h_bytes", "shk_set_upload_mode", "shk_upload_stats",
     "shk_reads_submit_packed", "shk_reads_upload_packed", "shk_result_expand", "shk_index_export_wide", "shk_reads_scores",
-    "shk_gene_counts", "shk_gene_counts_reset",
+    "shk_gene_counts", "shk_gene_counts_reset", "shk_eq_classes",
 ]
 
 
@@ -44,6 +44,7 @@ class Params(C.Structure):
 
 
 F_EXTEND_ON, F_EXTEND_OFF, F_HOST_PACK, F_COMPACT_RESULTS, F_WIDE_IDS, F_SCORES, F_GENE_COUNTS = 1, 2, 4, 8, 16, 32, 128
+F_EQ_CLASSES = 512
 GENE_NONE, GENE_MULTI = 0xFFFF, 0xFFFE
 
 
@@ -122,6 +123,7 @@ def load():
     L.shk_reads_scores.argtypes = [vp, C.c_uint32, C.POINTER(C.POINTER(ReadScore)), C.POINTER(C.c_uint32)]
     L.shk_gene_counts.argtypes = [vp, vp, vp, C.c_uint32]
     L.shk_gene_counts_reset.argtypes = [vp]
+    L.shk_eq_classes.argtypes = [vp, vp, vp, vp, vp, vp, C.c_uint64, C.c_uint64]
     L.shk_reads_upload.argtypes = [vp, C.c_uint32, vp, vp, vp, C.c_uint32]
     L.shk_reads_analyze_resident.argtypes = [vp, C.c_uint32]
     L.shk_device_timer_start.argtypes = [vp]

@@ -12,7 +12,11 @@
 // --scores FILE (one line `<name> <len> <cov> <hits> <n_best>` per reported read, in the order of the ssv: the numbers
 // behind each answer, from which any -c / -s can be applied afterwards - shk_read_score, include/shark_b200.h),
 // --counts FILE (one line `<name> <unique> <shared>` per gene index, in index order: the run's reported reads counted
-// per gene on the device - shk_gene_counts, include/shark_b200.h; <name> is the ssv's name of that index).
+// per gene on the device - shk_gene_counts, include/shark_b200.h; <name> is the ssv's name of that index),
+// --eqclasses FILE (one line `<count> <name_1> ... <name_n>` per equivalence class: the set of genes a reported read
+// is associated with, and the number of reads with exactly that set, counted on the device and summed over the GPUs -
+// shk_eq_classes, include/shark_b200.h; in lexicographic order of the ascending index lists, names as the ssv prints
+// them).
 //
 // Pipeline (pipeline.hpp, fastpipe.hpp, ingest.hpp): plain input files are memory-mapped and scanned by
 // the host pool in parallel (compressed ones by a streaming scanner per file); a batcher thread turns runs
@@ -48,6 +52,7 @@
 #include <vector>
 
 #include "../../../include/shark_b200.h"
+#include "eqclasses.hpp"
 #include "pipeline.hpp"
 
 namespace {
@@ -89,6 +94,7 @@ struct Options {
     std::string save_index, load_index;  // extensions
     std::string scores_path;        // extension: per-read score records (SHK_F_SCORES)
     std::string counts_path;        // extension: per-gene read counts (SHK_F_GENE_COUNTS)
+    std::string eqclasses_path;     // extension: reads per equivalence class (SHK_F_EQ_CLASSES)
 };
 
 [[noreturn]] void usage_error(const char *msg, bool with_usage)
@@ -162,6 +168,7 @@ const OptionRow kOptions[] = {
     {1005, "wide-ids", false, [](Options &o, std::istringstream &) { o.wide_ids = true; }},
     {1006, "scores", true, [](Options &o, std::istringstream &a) { a >> o.scores_path; }},
     {1007, "counts", true, [](Options &o, std::istringstream &a) { a >> o.counts_path; }},
+    {1008, "eqclasses", true, [](Options &o, std::istringstream &a) { a >> o.eqclasses_path; }},
 };
 
 Options parse_arguments(int argc, char **argv)
@@ -298,7 +305,8 @@ private:
 // list for ties, and with --scores the score records, 16 bytes per read; device -> host).  With --counts one more
 // region after the slots receives the per-gene table of the whole run (device -> host, once, before kMsgDone): it is
 // sized for the largest gene index count the run can have, 65536 (16-bit ids) or kMaxCountGenes (--wide-ids), and a
-// reference with more fails before the first chunk.  Two pipes carry the small messages.  SHK_ONE_PROCESS=1 runs the
+// reference with more fails before the first chunk.  The --eqclasses table, whose size is known only at the end, follows
+// the last result on the pipe (kMsgEqClasses, then its three arrays).  Two pipes carry the small messages.  SHK_ONE_PROCESS=1 runs the
 // device side as a thread of the host process instead (same protocol; for debuggers and sanitizers).
 // ---------------------------------------------------------------------------------------------------------
 struct SlotView {
@@ -352,11 +360,12 @@ struct SharedLayout {
     uint64_t *counts() const { return (uint64_t *)(base + n_slots * slot_bytes); }
 };
 
-enum : uint32_t { kMsgChunk = 1, kMsgEnd = 2, kMsgReady = 3, kMsgResult = 4, kMsgDone = 5 };
+enum : uint32_t { kMsgChunk = 1, kMsgEnd = 2, kMsgReady = 3, kMsgResult = 4, kMsgDone = 5, kMsgEqClasses = 6 };
 struct Msg {  // both directions; well below PIPE_BUF, so a write is atomic
     uint32_t kind = 0, slot = 0;
     uint32_t n_reads = 0, n_genes = 0;
     uint64_t n_bytes = 0, n_multi = 0, tail = 0;  // tail: multi entries that follow on the pipe (beyond the slot's capacity)
+                                                  // kMsgEqClasses: n_multi classes, tail ids
 };
 
 bool write_all(int fd, const void *p, size_t n)
@@ -435,7 +444,8 @@ void device_main(const Options &opt, const SharedLayout &shm, unsigned chunk_rea
         p.max_reads_per_chunk = chunk_reads;
         p.max_bytes_per_chunk = max_chunk_bytes;
         p.flags = SHK_F_COMPACT_RESULTS | (opt.wide_ids ? SHK_F_WIDE_IDS : 0u) | (opt.scores_path.empty() ? 0u : SHK_F_SCORES) |
-                  (shm.counts_cap ? SHK_F_GENE_COUNTS : 0u);
+                  (shm.counts_cap ? SHK_F_GENE_COUNTS : 0u) |
+                  (opt.eqclasses_path.empty() ? 0u : SHK_F_GENE_COUNTS | SHK_F_EQ_CLASSES);
         if (shk_create(&p, &ctxs[g]) != SHK_OK) die(std::string("shk_create: ") + shk_last_error(nullptr));
     }
     tstamp("contexts created");
@@ -531,6 +541,25 @@ void device_main(const Options &opt, const SharedLayout &shm, unsigned chunk_rea
             SHK_TRY(c, shk_gene_counts(c, u.data(), s.data(), n));
             for (uint32_t g = 0; g < n; ++g) tab[g] += u[g], tab[n + g] += s[g];
         }
+    }
+    if (!opt.eqclasses_path.empty()) {  // --eqclasses: the contexts' tables merged, length-prefixed on the pipe
+        std::vector<shkhost::EqTable> per(ctxs.size());
+        for (size_t g = 0; g < ctxs.size(); ++g) {
+            uint64_t n = 0, m = 0;
+            SHK_TRY(ctxs[g], shk_eq_classes(ctxs[g], &n, &m, nullptr, nullptr, nullptr, 0, 0));
+            per[g].offsets.resize(n + 1);
+            per[g].ids.resize(m);
+            per[g].counts.resize(n);
+            SHK_TRY(ctxs[g], shk_eq_classes(ctxs[g], &n, &m, per[g].offsets.data(), per[g].ids.data(), per[g].counts.data(), n, m));
+        }
+        const shkhost::EqTable t = shkhost::eq_merge(per);
+        Msg e;
+        e.kind = kMsgEqClasses;
+        e.n_multi = t.size();
+        e.tail = t.ids.size();
+        if (!write_all(out, &e, sizeof e) || !write_all(out, t.offsets.data(), t.offsets.size() * 8) ||
+            !write_all(out, t.ids.data(), t.ids.size() * 4) || !write_all(out, t.counts.data(), t.counts.size() * 8))
+            _exit(EXIT_FAILURE);
     }
     if (g_timing) fprintf(stderr, "[shark-b200/timing] device side: %llu chunks, submit %.0f ms, collect %.0f ms\n",
                           (unsigned long long)submitted, t_submit * 1e3, t_collect * 1e3);
@@ -692,6 +721,8 @@ int main(int argc, char *argv[])
     if (!opt.scores_path.empty() && fd_scores < 0) die("cannot create " + opt.scores_path);
     const int fd_counts = opt.counts_path.empty() ? -1 : open(opt.counts_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0666);
     if (!opt.counts_path.empty() && fd_counts < 0) die("cannot create " + opt.counts_path);
+    const int fd_eq = opt.eqclasses_path.empty() ? -1 : open(opt.eqclasses_path.c_str(), O_WRONLY | O_CREAT | O_TRUNC, 0666);
+    if (!opt.eqclasses_path.empty() && fd_eq < 0) die("cannot create " + opt.eqclasses_path);
     Writer writer(STDOUT_FILENO, fd1, fd2, legend_ID, opt.paired, fd_scores);
     if (!(getenv("SHK_PREFAULT") && atoi(getenv("SHK_PREFAULT")) == 0)) {
         // the filtered FASTQ of a FASTQ sample is never longer than the sample (pipeline.hpp, Writer::start_prefault)
@@ -716,7 +747,8 @@ int main(int argc, char *argv[])
     // results, in the order the chunks were sent
     uint64_t total_reads = 0, chunks_done = 0;
     uint32_t n_genes = 0;
-    bool got_ready = false, got_done = false;
+    bool got_ready = false, got_done = false, got_eq = false;
+    shkhost::EqTable eq;
     for (;;) {
         Msg m;
         if (!read_all(d2h[0], &m, sizeof m)) break;
@@ -726,6 +758,16 @@ int main(int argc, char *argv[])
             pelapsed("First switch performed");
             pelapsed("BF created from transcripts (" + std::to_string(m.n_genes) + " genes)");
             pelapsed("Second switch performed");
+            continue;
+        }
+        if (m.kind == kMsgEqClasses) {
+            eq.offsets.resize((size_t)m.n_multi + 1);
+            eq.ids.resize((size_t)m.tail);
+            eq.counts.resize((size_t)m.n_multi);
+            if (!read_all(d2h[0], eq.offsets.data(), eq.offsets.size() * 8) || !read_all(d2h[0], eq.ids.data(), eq.ids.size() * 4) ||
+                !read_all(d2h[0], eq.counts.data(), eq.counts.size() * 8))
+                break;
+            got_eq = true;
             continue;
         }
         if (m.kind == kMsgDone) {
@@ -751,7 +793,7 @@ int main(int argc, char *argv[])
         ++chunks_done;
         write_q.push(ch);
     }
-    if (!got_ready || !got_done) {
+    if (!got_ready || !got_done || (fd_eq >= 0 && !got_eq)) {
         fflush(nullptr);
         _exit(device_failed());
     }
@@ -774,6 +816,10 @@ int main(int argc, char *argv[])
             txt += '\n';
         }
         if (!write_all(fd_counts, txt.data(), txt.size()) || close(fd_counts) != 0) die("cannot write " + opt.counts_path);
+    }
+    if (fd_eq >= 0) {
+        const std::string txt = shkhost::eq_format(eq, legend_ID);
+        if (!write_all(fd_eq, txt.data(), txt.size()) || close(fd_eq) != 0) die("cannot write " + opt.eqclasses_path);
     }
     tstamp("output written");
     if (g_timing) {

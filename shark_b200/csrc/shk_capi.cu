@@ -63,6 +63,10 @@ static void free_slot(Slot &s)
     cudaFree(s.d_pack);
     cudaFree(s.d_scores);
     cudaFreeHost(s.h_scores);
+    cudaFree(s.d_eq_left);
+    cudaFree(s.d_eq_nleft);
+    cudaFreeHost(s.h_eq_nleft);
+    if (s.ev_eq) cudaEventDestroy(s.ev_eq);
     if (s.ev_start) cudaEventDestroy(s.ev_start);
     if (s.ev_k0) cudaEventDestroy(s.ev_k0);
     if (s.ev_ka) cudaEventDestroy(s.ev_ka);
@@ -205,6 +209,12 @@ static int alloc_slot(shk_ctx *ctx, Slot &s)
         SHK_CUDA(ctx, cudaMalloc((void **)&s.d_scores, R * sizeof(uint4)));
         SHK_CUDA(ctx, pinned_alloc((void **)&s.h_scores, R * sizeof(shk_read_score)));
     }
+    if (ctx->eq_classes) {
+        SHK_CUDA(ctx, cudaMalloc((void **)&s.d_eq_left, 2 * R * 4));
+        SHK_CUDA(ctx, cudaMalloc((void **)&s.d_eq_nleft, 2 * 4));
+        SHK_CUDA(ctx, pinned_alloc((void **)&s.h_eq_nleft, 4));
+        SHK_CUDA(ctx, cudaEventCreateWithFlags(&s.ev_eq, cudaEventDisableTiming));
+    }
     // packed reads: + 2 groups so that the kernels' prefetch of the following group stays inside
     s.pack_groups_cap = (B + 31) / 32 + 2;
     SHK_CUDA(ctx, cudaMalloc((void **)&s.d_pack, s.pack_groups_cap * 12));
@@ -270,6 +280,10 @@ static ReadKernelArgs make_args(shk_ctx *ctx, Slot &s)
     return a;
 }
 
+// SHK_F_EQ_CLASSES: the class table of a new index (growth doubles both)
+constexpr uint32_t kEqInitSlots = 4096;
+constexpr uint64_t kEqInitIds = 64 * 1024;
+
 // The exact-path tables depend on the number of gene indices -> (re)allocated after a build,
 // one set per slot because the slots' kernels run concurrently.
 static int ensure_slow_table(shk_ctx *ctx)
@@ -298,13 +312,18 @@ static int ensure_slow_table(shk_ctx *ctx)
         SHK_CUDA(ctx, cudaMemsetAsync(ctx->d_gene_counts, 0, 2 * ng * sizeof(unsigned long long), ctx->build_stream));
         SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
     }
+    if (ctx->eq_classes) {  // and so does the class table, at its initial size
+        std::lock_guard<std::mutex> lk(ctx->eq_mu);
+        if (int rc = eq_alloc(ctx, kEqInitSlots, kEqInitIds)) return rc;
+    }
     return SHK_OK;
 }
 
-// shk_gene_counts / shk_gene_counts_reset: the counters exist and no chunk is adding to them
-static int gene_counts_guard(shk_ctx *ctx)
+// shk_gene_counts / shk_gene_counts_reset / shk_eq_classes: the counters exist and no chunk is adding to them
+static int gene_counts_guard(shk_ctx *ctx, bool eq = false)
 {
     if (!ctx) return fail(nullptr, SHK_E_ARG, "NULL context");
+    if (eq && !ctx->eq_classes) return fail(ctx, SHK_E_STATE, "the context was created without SHK_F_EQ_CLASSES");
     if (!ctx->gene_counts) return fail(ctx, SHK_E_STATE, "the context was created without SHK_F_GENE_COUNTS");
     if (!ctx->index.built || !ctx->d_gene_counts) return fail(ctx, SHK_E_STATE, "no index");
     for (uint32_t i = 0; i < ctx->n_slots; ++i)
@@ -317,10 +336,17 @@ static int enqueue_chunk_kernels(shk_ctx *ctx, Slot &s)
 {
     s.collected = false;
     SHK_CUDA(ctx, cudaMemsetAsync(s.d_counters, 0, sizeof(ChunkCounters), s.stream));
+    if (ctx->eq_classes) SHK_CUDA(ctx, cudaMemsetAsync(s.d_eq_nleft, 0, 4, s.stream));
     ReadKernelArgs a = make_args(ctx, s);
-    s.launches += (uint32_t)launch_read_kernels(ctx, a, s.multi_cap, s.stream, s.ev_k0, s.ev_ka, s.ev_k1);
+    const EqPass eq{s.d_eq_left, s.d_eq_nleft, s.ev_eq};
+    s.launches += (uint32_t)launch_read_kernels(ctx, a, s.multi_cap, s.stream, s.ev_k0, s.ev_ka, s.ev_k1,
+                                                ctx->eq_classes ? &eq : nullptr);
     SHK_CUDA(ctx, cudaGetLastError());
     SHK_CUDA(ctx, cudaMemcpyAsync(s.h_counters, s.d_counters, sizeof(ChunkCounters), cudaMemcpyDeviceToHost, s.stream));
+    if (ctx->eq_classes) {  // the reads K8 left over: shk_reads_collect inserts them
+        SHK_CUDA(ctx, cudaMemcpyAsync(s.h_eq_nleft, s.d_eq_nleft, 4, cudaMemcpyDeviceToHost, s.stream));
+        ctx->d2h_bytes += 4;
+    }
     // Results follow on the stream, before the host knows their size: the per-read words, and as many multi
     // entries as the previous chunks produced per read (+10 %); the rest - if any - is fetched by
     // shk_reads_collect.  This keeps the read-back off the collecting thread's critical path and lets it
@@ -516,8 +542,10 @@ int shk_create(const shk_params *p, shk_ctx **out)
     if ((p->flags & SHK_F_EXTEND_ON) && (p->flags & SHK_F_EXTEND_OFF))
         return fail(nullptr, SHK_E_ARG, "SHK_F_EXTEND_ON and SHK_F_EXTEND_OFF are exclusive");
     if (p->flags & ~(SHK_F_EXTEND_ON | SHK_F_EXTEND_OFF | SHK_F_HOST_PACK | SHK_F_COMPACT_RESULTS | SHK_F_WIDE_IDS | SHK_F_SCORES |
-                     SHK_F_GENE_COUNTS))
+                     SHK_F_GENE_COUNTS | SHK_F_EQ_CLASSES))
         return fail(nullptr, SHK_E_ARG, "unknown flag bits");
+    if ((p->flags & SHK_F_EQ_CLASSES) && !(p->flags & SHK_F_GENE_COUNTS))
+        return fail(nullptr, SHK_E_ARG, "SHK_F_EQ_CLASSES needs SHK_F_GENE_COUNTS (its singleton classes are the gene counts)");
     if ((p->flags & SHK_F_WIDE_IDS) && (p->flags & SHK_F_EXTEND_ON))
         return fail(nullptr, SHK_E_ARG, "SHK_F_WIDE_IDS has no extension structures (SHK_F_EXTEND_ON)");
     const uint64_t n_words = (p->bf_bits + 31) / 32;
@@ -542,6 +570,11 @@ int shk_create(const shk_params *p, shk_ctx **out)
     ctx->wide_ids = (p->flags & SHK_F_WIDE_IDS) != 0;
     ctx->scores = (p->flags & SHK_F_SCORES) != 0;
     ctx->gene_counts = (p->flags & SHK_F_GENE_COUNTS) != 0;
+    ctx->eq_classes = (p->flags & SHK_F_EQ_CLASSES) != 0;
+    if (const char *ev = getenv("SHK_EQ_HASH_BITS")) {  // test knob: equal hashes of unequal class lists
+        const int bits = atoi(ev);
+        if (bits >= 0 && bits < 64) ctx->eq.hash_mask = (1ull << bits) - 1;
+    }
     if (const char *ev = getenv("SHK_HOST_PACK")) ctx->host_pack = atoi(ev) != 0;  // tuning override
     int rc = SHK_OK;
     auto bail = [&](int code) {
@@ -621,6 +654,10 @@ void shk_destroy(shk_ctx *ctx)
     cudaFree(ctx->index.ebits);
     cudaFree(ctx->index.front_plain);
     cudaFree(ctx->d_gene_counts);
+    cudaFree(ctx->eq.slots);
+    cudaFree(ctx->eq.count);
+    cudaFree(ctx->eq.arena);
+    cudaFree(ctx->eq.used);
     if (ctx->build_stream) cudaStreamDestroy(ctx->build_stream);
     if (ctx->ev_t0) cudaEventDestroy(ctx->ev_t0);
     if (ctx->ev_t1) cudaEventDestroy(ctx->ev_t1);
@@ -1194,6 +1231,41 @@ int shk_result_expand(const shk_chunk_result *res, shk_assoc *assoc, uint8_t *ke
     return SHK_OK;
 }
 
+// SHK_F_EQ_CLASSES: inserts the reads the chunk's K8 left over, without a probe limit, and never runs K8's counting
+// again.  Each pass first waits, without the lock, for the insert passes enqueued so far on every slot, so that the
+// slots they claimed are published.  Under the lock it grows the table when a claim was refused, no free slot was
+// found, or the reserved slots reach the load limit; growth waits for those passes once more, under the lock, since a
+// submit on another thread may have enqueued one meanwhile.  Submits of other slots block only while the lock is held.
+static int eq_finish(shk_ctx *ctx, Slot &s)
+{
+    uint32_t n = *s.h_eq_nleft, half = 0;
+    const ReadKernelArgs a = make_args(ctx, s);
+    for (int attempt = 0; n; ++attempt) {
+        if (attempt >= 64) return fail(ctx, SHK_E_STATE, "class table: %u reads still left over after 64 passes", n);
+        for (uint32_t i = 0; i < ctx->n_slots; ++i) SHK_CUDA(ctx, cudaEventSynchronize(ctx->slots[i].ev_eq));
+        {
+            std::lock_guard<std::mutex> lk(ctx->eq_mu);
+            unsigned long long used[3] = {0, 0, 0};
+            SHK_CUDA(ctx, cudaMemcpyAsync(used, ctx->eq.used, sizeof used, cudaMemcpyDeviceToHost, ctx->build_stream));
+            SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
+            if (used[2] || used[1] >= (unsigned long long)ctx->eq.cap / 4 * 3) {
+                if (int rc = eq_grow(ctx)) return rc;
+                s.launches += 1;
+            }
+            const EqPass out{s.d_eq_left + (size_t)(half ^ 1) * ctx->max_reads, s.d_eq_nleft + (half ^ 1), s.ev_eq};
+            SHK_CUDA(ctx, cudaMemsetAsync(out.n_left, 0, 4, s.stream));
+            if (int rc = eq_leftover_pass(ctx, a, s.d_eq_left + (size_t)half * ctx->max_reads, n, out, s.stream)) return rc;
+            s.launches += 1;
+            SHK_CUDA(ctx, cudaMemcpyAsync(s.h_eq_nleft, out.n_left, 4, cudaMemcpyDeviceToHost, s.stream));
+            ctx->d2h_bytes += 4;
+        }
+        SHK_CUDA(ctx, cudaStreamSynchronize(s.stream));
+        n = *s.h_eq_nleft;
+        half ^= 1;
+    }
+    return SHK_OK;
+}
+
 int shk_reads_collect(shk_ctx *ctx, uint32_t slot, shk_chunk_result *out)
 {
     if (!ctx || slot >= ctx->n_slots || !out) return fail(ctx, SHK_E_ARG, "bad argument");
@@ -1232,6 +1304,10 @@ int shk_reads_collect(shk_ctx *ctx, uint32_t slot, shk_chunk_result *out)
             continue;
         }
         break;
+    }
+    if (ctx->eq_classes && *s.h_eq_nleft) {
+        int rc = eq_finish(ctx, s);
+        if (rc) return rc;
     }
     const ChunkCounters c = *s.h_counters;
     if (c.n_multi > s.h_multi_cap) {
@@ -1325,6 +1401,73 @@ int shk_gene_counts_reset(shk_ctx *ctx)
     const uint64_t ng = std::max<uint32_t>(ctx->index.info.n_genes, 1);
     SHK_CUDA(ctx, cudaMemsetAsync(ctx->d_gene_counts, 0, 2 * ng * sizeof(unsigned long long), ctx->build_stream));
     SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
+    if (ctx->eq_classes) {  // the class table's singletons are these counters: it empties with them
+        std::lock_guard<std::mutex> lk(ctx->eq_mu);
+        if (int rc = eq_alloc(ctx, ctx->eq.cap, ctx->eq.arena_cap)) return rc;
+    }
+    return SHK_OK;
+}
+
+int shk_eq_classes(shk_ctx *ctx, uint64_t *n_classes, uint64_t *n_ids, uint64_t *offsets, uint32_t *ids, uint64_t *counts,
+                   uint64_t cap_classes, uint64_t cap_ids)
+{
+    int rc = gene_counts_guard(ctx, true);
+    if (rc) return rc;
+    if (!n_classes || !n_ids) return fail(ctx, SHK_E_ARG, "n_classes / n_ids is NULL");
+    const bool sizes_only = !offsets && !ids && !counts;
+    const uint32_t ng = ctx->index.info.n_genes;
+    const EqTable &t = ctx->eq;
+    std::vector<uint64_t> unique(ng), count(t.cap), used(3);
+    std::vector<EqSlot> slots(t.cap);
+    cudaStream_t st = ctx->build_stream;
+    if (ng) SHK_CUDA(ctx, cudaMemcpyAsync(unique.data(), ctx->d_gene_counts, (size_t)ng * 8, cudaMemcpyDeviceToHost, st));
+    SHK_CUDA(ctx, cudaMemcpyAsync(slots.data(), t.slots, (size_t)t.cap * sizeof(EqSlot), cudaMemcpyDeviceToHost, st));
+    SHK_CUDA(ctx, cudaMemcpyAsync(count.data(), t.count, (size_t)t.cap * 8, cudaMemcpyDeviceToHost, st));
+    SHK_CUDA(ctx, cudaMemcpyAsync(used.data(), t.used, 3 * 8, cudaMemcpyDeviceToHost, st));
+    SHK_CUDA(ctx, cudaStreamSynchronize(st));
+    const uint64_t n_arena = std::min<uint64_t>(used[0], t.arena_cap);
+    std::vector<uint32_t> arena(n_arena);
+    if (n_arena) SHK_CUDA(ctx, cudaMemcpyAsync(arena.data(), t.arena, n_arena * 4, cudaMemcpyDeviceToHost, st));
+    SHK_CUDA(ctx, cudaStreamSynchronize(st));
+    ctx->d2h_bytes += (uint64_t)ng * 8 + (uint64_t)t.cap * (sizeof(EqSlot) + 8) + 3 * 8 + n_arena * 4;
+    // every class as {first id, length, count}: singletons point into `single`, the table's lists into the arena
+    struct Cls {
+        const uint32_t *p;
+        uint32_t n;
+        uint64_t count;
+    };
+    std::vector<uint32_t> single(ng);
+    std::vector<Cls> cls;
+    for (uint32_t g = 0; g < ng; ++g) {
+        single[g] = g;
+        if (unique[g]) cls.push_back({&single[g], 1, unique[g]});
+    }
+    for (uint32_t j = 0; j < t.cap; ++j) {
+        if (!slots[j].len || !count[j]) continue;
+        if ((uint64_t)slots[j].off + slots[j].len > n_arena) return fail(ctx, SHK_E_STATE, "class table slot %u is corrupt", j);
+        cls.push_back({arena.data() + slots[j].off, slots[j].len, count[j]});
+    }
+    std::sort(cls.begin(), cls.end(), [](const Cls &x, const Cls &y) {
+        return std::lexicographical_compare(x.p, x.p + x.n, y.p, y.p + y.n);
+    });
+    uint64_t m = 0;
+    for (const Cls &c : cls) m += c.n;
+    *n_classes = cls.size();
+    *n_ids = m;
+    if (sizes_only) return SHK_OK;
+    if (!offsets || (m && !ids) || (!cls.empty() && !counts))
+        return fail(ctx, SHK_E_ARG, "offsets, ids and counts must all be given (ids and counts may be NULL when empty)");
+    if (cap_classes < cls.size() || cap_ids < m)
+        return fail(ctx, SHK_E_CAPACITY, "the table has %zu classes and %llu ids; the arrays hold %llu and %llu", cls.size(),
+                    (unsigned long long)m, (unsigned long long)cap_classes, (unsigned long long)cap_ids);
+    uint64_t o = 0;
+    for (size_t i = 0; i < cls.size(); ++i) {
+        offsets[i] = o;
+        memcpy(ids + o, cls[i].p, (size_t)cls[i].n * 4);
+        o += cls[i].n;
+        counts[i] = cls[i].count;
+    }
+    offsets[cls.size()] = o;
     return SHK_OK;
 }
 

@@ -6,6 +6,7 @@
 #include <cstdarg>
 #include <cstdint>
 #include <cstdio>
+#include <mutex>
 #include <string>
 
 #include "../../include/shark_b200.h"
@@ -117,6 +118,32 @@ struct ReadKernelArgs {
     uint4 *scores;
 };
 
+// SHK_F_EQ_CLASSES: a device hash table from the id list of a tied read (n_best >= 2) to the number of reads with that
+// list; singletons are the gene counts' `unique`.  A slot is empty while hash == 0 (list hashes are never 0), claimed by
+// the CAS that sets hash, and published once len != 0 (release store after off and the arena ids).
+struct EqSlot {
+    unsigned long long hash;
+    uint32_t off;  // first id in the arena
+    uint32_t len;  // 0 until published
+};
+struct EqTable {
+    EqSlot *slots = nullptr;              // cap (a power of two)
+    unsigned long long *count = nullptr;  // cap: reads per slot
+    uint32_t *arena = nullptr;            // arena_cap ids
+    // [0] arena ids reserved, [1] slots reserved for claims (at least those claimed), [2] != 0: a claim was refused for
+    // the load limit or a full arena, or a pass without a probe limit found no free slot: the table must grow
+    unsigned long long *used = nullptr;
+    uint32_t cap = 0;
+    uint64_t arena_cap = 0;
+    unsigned long long hash_mask = ~0ull;  // SHK_EQ_HASH_BITS (tests): the list hash keeps only these bits
+};
+// where an insert pass parks the reads it could not place (slot-private), and the event after it
+struct EqPass {
+    uint32_t *left;
+    uint32_t *n_left;
+    cudaEvent_t ev;
+};
+
 constexpr uint32_t kReadsPerTile = 128;  // one CTA of the fast kernel: 128 threads = 128 reads
 constexpr uint32_t kDerivedPad = 2;     // zero words in front of refr / ebits (a read may overhang the reference)
 constexpr uint32_t kDerivedTail = 4;    // and behind
@@ -157,6 +184,10 @@ struct Slot {
     // SHK_F_SCORES only: one record per read, read back with the other results
     uint4 *d_scores = nullptr;
     shk_read_score *h_scores = nullptr;
+    // SHK_F_EQ_CLASSES only: reads the insert passes left over (two halves of max_reads: a leftover pass reads one and
+    // writes the other), their counts, the count read back with the chunk, and the event after the slot's last insert
+    uint32_t *d_eq_left = nullptr, *d_eq_nleft = nullptr, *h_eq_nleft = nullptr;
+    cudaEvent_t ev_eq = nullptr;
     // state
     uint32_t n_reads = 0;
     uint64_t n_bytes = 0;
@@ -226,6 +257,10 @@ struct shk_ctx {
     // SHK_F_GENE_COUNTS: [0, n_genes) reads whose only association is g, [n_genes, 2 n_genes) reads with g among tied
     // associations; (re)allocated and zeroed whenever an index becomes ready, added to by every chunk's K8
     unsigned long long *d_gene_counts = nullptr;
+    bool eq_classes = false;               // SHK_F_EQ_CLASSES
+    shk::EqTable eq;                       // (re)allocated at its initial size whenever an index becomes ready
+    // taken by every enqueue of an insert pass and by growth, which frees the table those passes were given
+    std::mutex eq_mu;
     shk::PackControl pack;                 // split upload: feedback state of the packed share
     char err[512] = {0};
 };
@@ -270,10 +305,17 @@ void shard_free(shk_ctx *ctx);
 void shard_cuts_host(const uint64_t *rec_off, uint32_t n_rec, uint32_t n_shards, uint64_t *cuts);
 
 // shk_reads.cu
-// Enqueues the classification kernels of one chunk on `st` (and K8 when ctx->d_gene_counts exists); returns the number
-// of launches.
+// Enqueues the classification kernels of one chunk on `st` (and K8 when ctx->d_gene_counts exists, with the insert pass
+// of SHK_F_EQ_CLASSES when `eq` is given); returns the number of launches.
 int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t assoc_cap, cudaStream_t st, cudaEvent_t ev_k0,
-                        cudaEvent_t ev_ka, cudaEvent_t ev_k1);
+                        cudaEvent_t ev_ka, cudaEvent_t ev_k1, const EqPass *eq = nullptr);
+// SHK_F_EQ_CLASSES, with ctx->eq_mu held.  eq_alloc: an empty table (frees the old one).  eq_grow: once every insert pass
+// enqueued on any slot has finished, rehashes into a table twice the size.  eq_leftover_pass: inserts n_in reads of the
+// list `in` (rec / pool of a settled chunk) without a probe limit; reads it cannot place go to `out`.
+int eq_alloc(shk_ctx *ctx, uint32_t cap, uint64_t arena_cap);
+int eq_grow(shk_ctx *ctx);
+int eq_leftover_pass(shk_ctx *ctx, const ReadKernelArgs &a, const uint32_t *in, uint32_t n_in, const EqPass &out,
+                     cudaStream_t st);
 int launch_scatter(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t assoc_cap, cudaStream_t st);
 // shk_bulk.cu: the bulk classification kernel for packed reads over the extension structures
 bool bulk_enabled();

@@ -14,7 +14,10 @@
 //   scan_tile_sums_kernel  exclusive scan of the per-tile association counts
 //   scatter_assoc_kernel   ordered (read_idx, gene_idx) list + keep flags
 //   gene_counts_kernel     K8, SHK_F_GENE_COUNTS only: per-gene counts of the chunk's reported reads, added into the
-//                          context's device counters
+//                          context's device counters; with EQ (SHK_F_EQ_CLASSES) it also inserts every tied read's
+//                          winner list into the context's class table
+//   eq_leftover_kernel     SHK_F_EQ_CLASSES: inserts the reads K8 left over, without a probe limit
+//   eq_rehash_kernel       SHK_F_EQ_CLASSES: moves the class table into one twice the size
 #include "shk_internal.h"
 #include "shk_scan.cuh"
 #include "shk_reads.cuh"
@@ -798,10 +801,115 @@ scatter_assoc_kernel(const ReadKernelArgs a, uint64_t multi_cap, const uint32_t 
 constexpr uint32_t kCountThreads = 256;
 constexpr uint32_t kCountSmemGenes = 6144;  // 2 x 6144 32-bit bins = 48 KB, the most static shared memory a kernel may have
 
-template <bool SMEM>
+// ---------------------------------------------------------------------------------------------
+// SHK_F_EQ_CLASSES: the class table (EqTable, shk_internal.h).  One warp inserts one id list: the lanes hash it
+// together, probe linearly from a slot the hash picks, and either add 1 to the slot whose published list equals theirs
+// (compared id by id: the hash only picks the slots to compare) or claim an empty slot.  A claimer reserves a slot
+// (used[1], refused at 3/4 of the slots, so in-flight claims never fill the table) and its arena range before the CAS,
+// so a claimed slot is always published: it writes the ids, then off, then len with release semantics.  A warp that
+// loses the CAS to a warp inserting the same new list adds to that slot, and its reservations stay unused until the
+// next growth compacts the arena: a burst of one new class arriving in many warps at once can use up the arena (or the
+// slot budget) and bring a growth forward that the live classes do not need.  No wait is unbounded: a warp that meets an unpublished slot with its hash polls it kEqSpins times and
+// then leaves the read over, as it does past kEqProbes slots (K8 only), at the load limit (3/4 of the slots) or with
+// the arena full.  Left-over reads go to a slot-private list; shk_reads_collect inserts them in later launches (after
+// a kernel boundary every claimed slot is published), growing the table first when a claim was refused.
+// ---------------------------------------------------------------------------------------------
+constexpr uint32_t kEqProbes = 64;
+constexpr uint32_t kEqSpins = 2048;
+constexpr uint32_t kEqThreads = 256;
+
+__device__ __forceinline__ unsigned long long eq_mix(unsigned long long x)  // splitmix64 finaliser
+{
+    x ^= x >> 30;
+    x *= 0xbf58476d1ce4e5b9ull;
+    x ^= x >> 27;
+    x *= 0x94d049bb133111ebull;
+    return x ^ (x >> 31);
+}
+
+__device__ __forceinline__ uint32_t eq_ld_acquire(const uint32_t *p)
+{
+    uint32_t v;
+    asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+
+__device__ __forceinline__ void eq_st_release(uint32_t *p, uint32_t v)
+{
+    asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+
+// Warp-collective; every lane gets the same answer: 0 placed, 1 left over, 2 left over and the table must grow.
+__device__ __noinline__ int eq_insert(const EqTable t, const uint32_t *__restrict__ ids, uint32_t n, uint32_t max_probes)
+{
+    const int lane = threadIdx.x & 31;
+    unsigned long long h = 0;
+    for (uint32_t i = lane; i < n; i += 32) h += eq_mix(((unsigned long long)i << 32 | ids[i]) + 0x9e3779b97f4a7c15ull);
+    for (int o = 16; o; o >>= 1) h += __shfl_xor_sync(kFull, h, o);
+    h = (eq_mix(h ^ n) & t.hash_mask) + 1u;  // never 0 (empty) unless the mask keeps all 64 bits
+    if (!h) h = 1;
+    const uint32_t mask = t.cap - 1u;
+    uint32_t j = (uint32_t)eq_mix(h) & mask;
+    unsigned long long res = ~0ull;  // arena range reserved for a claim
+    for (uint32_t p = 0; p < max_probes; ++p, j = (j + 1u) & mask) {
+        EqSlot *s = t.slots + j;
+        unsigned long long cur = 0;
+        if (lane == 0) cur = __ldcg(&s->hash);
+        cur = __shfl_sync(kFull, cur, 0);
+        if (cur == 0) {
+            if (res == ~0ull) {
+                int refused = 0;
+                if (lane == 0) {  // a slot and an arena range, both reserved before the CAS
+                    if (atomicAdd(&t.used[1], 1ull) >= (unsigned long long)t.cap / 4 * 3) refused = 1;
+                    else {
+                        res = atomicAdd(&t.used[0], (unsigned long long)n);
+                        if (res + n > t.arena_cap) refused = 1;
+                    }
+                    if (refused) atomicExch(&t.used[2], 1ull);
+                }
+                if (__shfl_sync(kFull, refused, 0)) return 2;
+                res = __shfl_sync(kFull, res, 0);
+            }
+            if (lane == 0) cur = atomicCAS(&s->hash, 0ull, h);
+            cur = __shfl_sync(kFull, cur, 0);
+            if (cur == 0) {  // claimed: publish
+                for (uint32_t i = lane; i < n; i += 32) t.arena[res + i] = ids[i];
+                __threadfence();
+                __syncwarp();
+                if (lane == 0) {
+                    s->off = (uint32_t)res;
+                    eq_st_release(&s->len, n);
+                    atomicAdd(&t.count[j], 1ull);
+                }
+                return 0;
+            }
+        }
+        if (cur != h) continue;
+        uint32_t len = 0;
+        if (lane == 0)
+            for (uint32_t w = 0; !(len = eq_ld_acquire(&s->len)) && w < kEqSpins; ++w) __nanosleep(128);
+        len = __shfl_sync(kFull, len, 0);
+        __syncwarp();
+        if (!len) return 1;  // still unpublished: a later launch inserts the read
+        if (len != n) continue;
+        const uint32_t off = __ldcg(&s->off);
+        bool same = true;
+        for (uint32_t i = lane; i < n; i += 32) same &= __ldcg(t.arena + off + i) == ids[i];
+        if (__all_sync(kFull, same)) {
+            if (lane == 0) atomicAdd(&t.count[j], 1ull);
+            return 0;
+        }
+    }
+    if (max_probes < t.cap) return 1;  // K8's probe limit: the leftover pass probes every slot
+    if (lane == 0) atomicExch(&t.used[2], 1ull);  // every slot probed, none free: only a larger table takes the read
+    return 2;
+}
+
+template <bool SMEM, bool EQ>
 __global__ void __launch_bounds__(kCountThreads)
 gene_counts_kernel(const uint2 *__restrict__ rec, const uint32_t *__restrict__ pool, uint32_t n_reads, uint32_t n_genes,
-                   const ChunkCounters *counters, unsigned long long *counts)
+                   const ChunkCounters *counters, unsigned long long *counts, const EqTable eq, uint32_t *left,
+                   uint32_t *n_left)
 {
     __shared__ uint32_t hist[SMEM ? 2 * kCountSmemGenes : 1];
     if (counters->pool_overflow) return;  // the same for every thread of the grid
@@ -824,6 +932,7 @@ gene_counts_kernel(const uint2 *__restrict__ rec, const uint32_t *__restrict__ p
             const int src = __ffs(tied) - 1;
             const uint32_t cnt = __shfl_sync(kFull, rc.x, src), off = __shfl_sync(kFull, rc.y, src);
             for (uint32_t t = lane; t < cnt; t += 32) add(n_genes + pool[off + t], 1u);
+            if (EQ && eq_insert(eq, pool + off, cnt, kEqProbes) && lane == 0) left[atomicAdd(n_left, 1u)] = w + src;
         }
     }
     if (SMEM) {
@@ -833,15 +942,116 @@ gene_counts_kernel(const uint2 *__restrict__ rec, const uint32_t *__restrict__ p
     }
 }
 
-static void launch_gene_counts(shk_ctx *ctx, const ReadKernelArgs &a, cudaStream_t st)
+template <bool EQ>
+static void launch_gene_counts(shk_ctx *ctx, const ReadKernelArgs &a, cudaStream_t st, const EqTable &t, const EqPass *eq)
 {
     const bool smem = a.n_genes <= kCountSmemGenes;
     const unsigned per_sm = smem ? 4u : 8u;
     const unsigned blocks = std::min<unsigned>((a.n_reads + kCountThreads - 1) / kCountThreads, (unsigned)ctx->sm_count * per_sm);
+    uint32_t *left = eq ? eq->left : nullptr, *n_left = eq ? eq->n_left : nullptr;
     if (smem)
-        gene_counts_kernel<true><<<blocks, kCountThreads, 0, st>>>(a.rec, a.pool, a.n_reads, a.n_genes, a.counters, ctx->d_gene_counts);
+        gene_counts_kernel<true, EQ><<<blocks, kCountThreads, 0, st>>>(a.rec, a.pool, a.n_reads, a.n_genes, a.counters,
+                                                                     ctx->d_gene_counts, t, left, n_left);
     else
-        gene_counts_kernel<false><<<blocks, kCountThreads, 0, st>>>(a.rec, a.pool, a.n_reads, a.n_genes, a.counters, ctx->d_gene_counts);
+        gene_counts_kernel<false, EQ><<<blocks, kCountThreads, 0, st>>>(a.rec, a.pool, a.n_reads, a.n_genes, a.counters,
+                                                                      ctx->d_gene_counts, t, left, n_left);
+}
+
+__global__ void __launch_bounds__(kEqThreads)
+eq_leftover_kernel(const uint2 *__restrict__ rec, const uint32_t *__restrict__ pool, const uint32_t *__restrict__ in,
+                   uint32_t n_in, const EqTable t, uint32_t *out, uint32_t *n_out)
+{
+    const int lane = threadIdx.x & 31;
+    for (uint32_t w = (blockIdx.x * kEqThreads + threadIdx.x) >> 5; w < n_in; w += gridDim.x * (kEqThreads / 32)) {
+        const uint32_t r = in[w];
+        const uint2 rc = rec[r];
+        if (eq_insert(t, pool + rc.y, rc.x, t.cap) && lane == 0) out[atomicAdd(n_out, 1u)] = r;
+    }
+}
+
+// One thread per slot of `from`; nothing else touches either table meanwhile, and every claimed slot is published.
+__global__ void __launch_bounds__(kEqThreads) eq_rehash_kernel(const EqTable from, const EqTable to)
+{
+    const uint32_t mask = to.cap - 1u;
+    for (uint32_t i = blockIdx.x * kEqThreads + threadIdx.x; i < from.cap; i += gridDim.x * kEqThreads) {
+        const EqSlot s = from.slots[i];
+        if (!s.len) continue;
+        const unsigned long long o = atomicAdd(&to.used[0], (unsigned long long)s.len);
+        for (uint32_t k = 0; k < s.len; ++k) to.arena[o + k] = from.arena[s.off + k];
+        uint32_t j = (uint32_t)eq_mix(s.hash) & mask;
+        while (atomicCAS(&to.slots[j].hash, 0ull, s.hash) != 0ull) j = (j + 1u) & mask;  // to.cap > live slots
+        to.slots[j].off = (uint32_t)o;
+        to.slots[j].len = s.len;
+        to.count[j] = from.count[i];
+        atomicAdd(&to.used[1], 1ull);
+    }
+}
+
+static void eq_free(EqTable &t)
+{
+    cudaFree(t.slots);
+    cudaFree(t.count);
+    cudaFree(t.arena);
+    cudaFree(t.used);
+    t.slots = nullptr, t.count = nullptr, t.arena = nullptr, t.used = nullptr;
+    t.cap = 0, t.arena_cap = 0;
+}
+
+static int eq_alloc_table(shk_ctx *ctx, EqTable &t, uint32_t cap, uint64_t arena_cap)
+{
+    SHK_CUDA(ctx, cudaMalloc((void **)&t.slots, (size_t)cap * sizeof(EqSlot)));
+    SHK_CUDA(ctx, cudaMalloc((void **)&t.count, (size_t)cap * 8));
+    SHK_CUDA(ctx, cudaMalloc((void **)&t.arena, arena_cap * 4));
+    SHK_CUDA(ctx, cudaMalloc((void **)&t.used, 3 * 8));
+    t.cap = cap;
+    t.arena_cap = arena_cap;
+    SHK_CUDA(ctx, cudaMemsetAsync(t.slots, 0, (size_t)cap * sizeof(EqSlot), ctx->build_stream));
+    SHK_CUDA(ctx, cudaMemsetAsync(t.count, 0, (size_t)cap * 8, ctx->build_stream));
+    SHK_CUDA(ctx, cudaMemsetAsync(t.used, 0, 3 * 8, ctx->build_stream));
+    return SHK_OK;
+}
+
+int eq_alloc(shk_ctx *ctx, uint32_t cap, uint64_t arena_cap)
+{
+    const unsigned long long mask = ctx->eq.hash_mask;
+    eq_free(ctx->eq);
+    ctx->eq.hash_mask = mask;
+    if (int rc = eq_alloc_table(ctx, ctx->eq, cap, arena_cap)) return rc;
+    SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
+    return SHK_OK;
+}
+
+int eq_grow(shk_ctx *ctx)
+{
+    for (uint32_t i = 0; i < ctx->n_slots; ++i) SHK_CUDA(ctx, cudaEventSynchronize(ctx->slots[i].ev_eq));
+    EqTable &from = ctx->eq;
+    if (from.cap >= (1u << 30) || from.arena_cap >= (1ull << 31))
+        return fail(ctx, SHK_E_LIMIT, "the class table would exceed 2^31 slots or 2^32 ids");
+    EqTable to;
+    to.hash_mask = from.hash_mask;
+    if (int rc = eq_alloc_table(ctx, to, from.cap * 2, from.arena_cap * 2)) {
+        eq_free(to);
+        return rc;
+    }
+    const unsigned blocks = std::min<unsigned>((from.cap + kEqThreads - 1) / kEqThreads, (unsigned)ctx->sm_count * 8);
+    eq_rehash_kernel<<<blocks, kEqThreads, 0, ctx->build_stream>>>(from, to);
+    SHK_CUDA(ctx, cudaGetLastError());
+    SHK_CUDA(ctx, cudaStreamSynchronize(ctx->build_stream));
+    eq_free(from);
+    ctx->eq = to;
+    ctx->launches += 1;
+    return SHK_OK;
+}
+
+int eq_leftover_pass(shk_ctx *ctx, const ReadKernelArgs &a, const uint32_t *in, uint32_t n_in, const EqPass &out,
+                     cudaStream_t st)
+{
+    const unsigned blocks = std::min<unsigned>((n_in + kEqThreads / 32 - 1) / (kEqThreads / 32), (unsigned)ctx->sm_count * 8);
+    eq_leftover_kernel<<<blocks, kEqThreads, 0, st>>>(a.rec, a.pool, in, n_in, ctx->eq, out.left, out.n_left);
+    SHK_CUDA(ctx, cudaGetLastError());
+    SHK_CUDA(ctx, cudaEventRecord(out.ev, st));
+    ctx->launches += 1;
+    return SHK_OK;
 }
 
 // SHK_F_WIDE_IDS: there is no front table, every read goes to the middle path.
@@ -911,7 +1121,7 @@ static void launch_classify(const ReadKernelArgs &a, cudaStream_t st, unsigned t
 }
 
 int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t multi_cap, cudaStream_t st, cudaEvent_t ev_k0,
-                        cudaEvent_t ev_ka, cudaEvent_t ev_k1)
+                        cudaEvent_t ev_ka, cudaEvent_t ev_k1, const EqPass *eq)
 {
     if (ev_k0) cudaEventRecord(ev_k0, st);
     int launched = 0;
@@ -921,7 +1131,13 @@ int launch_read_kernels(shk_ctx *ctx, const ReadKernelArgs &a, uint64_t multi_ca
         cudaMemsetAsync(a.tile_sums, 0, (size_t)tiles * 4, st);  // the classification kernels add to it
         if (a.scores) launch_classify<true>(a, st, tiles, slow_blocks, ev_ka);
         else launch_classify<false>(a, st, tiles, slow_blocks, ev_ka);
-        if (ctx->d_gene_counts) launch_gene_counts(ctx, a, st);
+        if (ctx->d_gene_counts && eq) {  // growth frees the table this launch is given
+            std::lock_guard<std::mutex> lk(ctx->eq_mu);
+            launch_gene_counts<true>(ctx, a, st, ctx->eq, eq);
+            cudaEventRecord(eq->ev, st);
+        } else if (ctx->d_gene_counts) {
+            launch_gene_counts<false>(ctx, a, st, EqTable{}, nullptr);
+        }
         // tile_base <- exclusive scan(tile_sums); the grand total lands in tile_base[tiles]
         cudaMemcpyAsync(a.tile_base, a.tile_sums, (size_t)tiles * 4, cudaMemcpyDeviceToDevice, st);
         scan_tile_sums_kernel<<<1, 1024, 0, st>>>(a.tile_base, tiles, a.tile_base + tiles);

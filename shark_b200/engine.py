@@ -16,13 +16,15 @@ from . import capi
 class Shark:
     def __init__(self, k=17, c=0.6, bf_bits=1 << 33, min_quality=0, single=False, device=0, n_slots=2,
                  max_reads_per_chunk=1 << 20, max_bytes_per_chunk=0, extend=None, host_pack=False, compact=False,
-                 wide_ids=False, scores=False, gene_counts=False):
+                 wide_ids=False, scores=False, gene_counts=False, eq_classes=False):
         """extend: None = automatic (anchor-and-extend when the front table is DRAM-sized), True /
         False = force it on / off (results are identical; tests run both).  compact: results stay in the
         compact form (gene16 / multi), shk_reads_collect does no per-read host work.  scores: every result also
         carries the per-read score records {len, cov, hits, n_best} (SHK_F_SCORES, include/shark_b200.h).
         gene_counts: every chunk's reported reads are also counted per gene on the device (SHK_F_GENE_COUNTS);
-        gene_counts() reads the table back."""
+        gene_counts() reads the table back.  eq_classes: the reported reads are also counted per equivalence class (the
+        set of genes a read is associated with) on the device (SHK_F_EQ_CLASSES, which needs and sets
+        SHK_F_GENE_COUNTS); eq_classes() reads the table back."""
         self.lib = capi.load()
         flags = 0 if extend is None else (capi.F_EXTEND_ON if extend else capi.F_EXTEND_OFF)
         if compact:
@@ -31,8 +33,10 @@ class Shark:
             flags |= capi.F_WIDE_IDS
         if scores:
             flags |= capi.F_SCORES
-        if gene_counts:
+        if gene_counts or eq_classes:
             flags |= capi.F_GENE_COUNTS
+        if eq_classes:
+            flags |= capi.F_EQ_CLASSES
         self.compact = bool(compact)
         self.scores = bool(scores)
         self.wide_ids = bool(wide_ids)
@@ -271,7 +275,22 @@ class Shark:
         return unique, shared
 
     def reset_gene_counts(self):
+        """Zeroes the gene counts; with eq_classes=True it also empties the class table (its singletons are the
+        counts)."""
         self._check(self.lib.shk_gene_counts_reset(self.ctx))
+
+    def eq_classes(self):
+        """-> (offsets uint64[n+1], ids uint32[m], counts uint64[n]): class i is ids[offsets[i]:offsets[i+1]], an
+        ascending gene id list, and counts[i] reported reads had exactly that set of associations, summed like
+        gene_counts().  Classes come in lexicographic order of their lists (Python's sorted on tuples), singletons
+        included (shk_eq_classes; needs eq_classes=True and every submitted chunk collected)."""
+        n, m = C.c_uint64(), C.c_uint64()
+        self._check(self.lib.shk_eq_classes(self.ctx, C.byref(n), C.byref(m), None, None, None, 0, 0))
+        offsets = np.zeros(n.value + 1, np.uint64)
+        ids, counts = np.zeros(max(m.value, 1), np.uint32)[:m.value], np.zeros(max(n.value, 1), np.uint64)[:n.value]
+        self._check(self.lib.shk_eq_classes(self.ctx, C.byref(n), C.byref(m), capi.ptr(offsets), capi.ptr(ids),
+                                            capi.ptr(counts), n.value, m.value))
+        return offsets, ids, counts
 
     def collect(self, slot, copy=True):
         """-> dict(read_idx, gene_idx, keep, gene16, multi, n_probes, n_hits, analyze_ms, ...); with compact=True
